@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N ...            # the reference's own CPU path on the host cores
+  python bench.py ... --dump-outputs DIR                   # + what the last timed step computed, as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of synthetic input (BASELINE.json config C0):
   images [64,3,641,641] f32 -> shufflenetv2k16 backbone + CIF/CAF heads -> batched CifCaf decode.
@@ -328,6 +329,29 @@ def extra_config(name, local, pk, steps=5, warmup=3):
         return {'error': f'{type(e).__name__}: {e}'[:300]}
 
 
+DUMP_HEAD_IMAGES = 16       # cif + caf of 16 images of 641 px: 25.5 MB of float32
+
+
+def dump_outputs(out_dir, results, heads):
+    """What the last timed step computed, as .npy files a second build's dump can be compared with: the decoded
+    annotations of every image (concatenated, with per-image counts and ids) and the two head outputs of a fixed,
+    seeded sample of DUMP_HEAD_IMAGES images (all heads of a 64-image batch would be 100 MB)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cif, caf = heads
+    b = int(cif.shape[0])
+    pick = np.sort(np.random.default_rng(0).choice(b, min(b, DUMP_HEAD_IMAGES), replace=False))
+    arrays = {
+        'annotations': np.concatenate([a.numpy() for a, _ in results]).astype(np.float32),
+        'annotation_counts': np.array([len(a) for a, _ in results], dtype=np.float64),
+        'annotation_ids': np.concatenate([i.numpy() for _, i in results]).astype(np.float64),
+        'head_images': pick.astype(np.float64),
+        'cif': cif[torch.from_numpy(pick).to(cif.device)].cpu().numpy().astype(np.float32),
+        'caf': caf[torch.from_numpy(pick).to(caf.device)].cpu().numpy().astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def load_committed(name):
     try:
         with open(os.path.join(ROOT, 'profiles', name)) as f:
@@ -373,9 +397,12 @@ def run_b200(args):
     ms_per_step = timed_steps(pred, dev_images, args.steps, 0, world, device)
     launches = int(_lib.lib().pifpaf_launch_count() - launches0)
     clocks = sampler.stop()
-    n_ann_value = sum(len(a) for a, _ in pred.decoder.fetch(stream=pred.result_stream()))
+    results = pred.decoder.fetch(stream=pred.result_stream())
+    n_ann_value = sum(len(a) for a, _ in results)
     torch.cuda.synchronize()
     value = world * B / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, results, net._head_views(B))
 
     # ---- end to end through the public API with host buffers: Predictor.batches() is the pipelined
     # iterator (H2D of batch i+1 under the compute of batch i), like the reference's Predictor.dataloader()
@@ -516,9 +543,8 @@ def reference_step_setup(cpu_sample):
     cfg = CONFIGS['C0']
     plan = make_plan(cfg)
     images = torch.randn((cpu_sample, 3, SIZE, SIZE), generator=torch.Generator().manual_seed(1234))
-    # head calibration like network.calibrate_random_heads, on the reference Shell's own features
-    op = ref_arm.import_reference()
-    shell = ref_arm.shell_from_plan(op, plan, cfg['base'], cfg['workload'])
+    # head calibration like network.calibrate_random_heads, on the CPU arm's own features
+    shell = ref_arm.cpu_shell(plan, cfg['base'], cfg['workload'])
     with torch.no_grad():     # the input network.calibrate_random_heads draws on the GPU side
         feat = shell.base_net(torch.randn((2, 3, SIZE, SIZE), generator=torch.Generator().manual_seed(0)))
     f = feat.permute(0, 2, 3, 1).reshape(-1, feat.shape[1]).double().numpy()
@@ -549,12 +575,8 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    from oracle import ref_arm
     base = {'metric': METRIC, 'unit': 'images/s', 'n_gpus': args.gpus, 'higher_is_better': True, 'scaling': 'strong',
             'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic', 'impl': 'reference', 'gpu_launches': 0}
-    if not ref_arm.available():
-        print(json.dumps(dict(base, unavailable='oracle/_ref_pkg (the staged reference package) is missing')), flush=True)
-        return
     sample = args.cpu_sample
     ref_arm_mod, plan, cfg, images, planted = reference_step_setup(sample)
     steps, warmup = max(1, args.steps), max(0, min(args.warmup, 2))
@@ -564,12 +586,20 @@ def run_reference(args):
     steps_run = int(max(1, min(steps, budget_s // max(probe['seconds'], 1e-3))))
     res = ref_arm_mod.run_cpu(plan, cfg['base'], cfg['workload'], images, planted, steps_run, 0)
     value = res['images'] / res['seconds']
-    desc = (f"{sample} images of the C0 batch per step, {steps_run} of {steps} steps (150 s budget): the reference's own "
-            f"Shell (network.Factory, same weights as the CUDA arm) on PyTorch-CPU fp32, {res['cores']} threads = the "
-            f"fastest of all / half / quarter / eighth of the {os.cpu_count()} host cores, + its Decoder.batch with the C++ "
-            f"CifCaf decoding the planted fields of the same images, serial per image (decoder/decoder.py:33-34); "
-            f"forward {res['nn_seconds'] / steps_run:.2f} s + decode {res['decoder_seconds'] / steps_run * 1e3:.1f} ms per step")
-    cpu = {'value': round(value, 3), 'unit': 'images/s', 'cores': res['cores'], 'kind': 'reference', 'sample': desc,
+    if res['kind'] == 'reference':
+        what = ("the reference's own Shell (network.Factory, same weights as the CUDA arm) on PyTorch-CPU fp32, "
+                "{threads}, + its Decoder.batch with the C++ CifCaf decoding the planted fields of the same images, "
+                "serial per image (decoder/decoder.py:33-34)")
+    else:
+        what = ("the port (the reference package is not staged): oracle/net_oracle.py's Shell (same weights as the "
+                "CUDA arm) on PyTorch-CPU fp32, {threads}, + the plain-C oracle CifCaf decoding the planted fields of "
+                "the same images, serial per image")
+    threads = (f"{res['cores']} threads = the fastest of all / half / quarter / eighth of the {os.cpu_count()} "
+               f"host cores")
+    desc = (f"{sample} images of the C0 batch per step, {steps_run} of {steps} steps (150 s budget): "
+            + what.format(threads=threads)
+            + f"; forward {res['nn_seconds'] / steps_run:.2f} s + decode {res['decoder_seconds'] / steps_run * 1e3:.1f} ms per step")
+    cpu = {'value': round(value, 3), 'unit': 'images/s', 'cores': res['cores'], 'kind': res['kind'], 'sample': desc,
            'annotations_last_step': res['annotations_last_step']}
     out = dict(base, value=round(value, 3), steps=steps_run, warmup=warmup,
                ms_per_step=round(res['seconds'] / steps_run * 1e3, 2),
@@ -596,6 +626,8 @@ def main():
     ap.add_argument('--raw-input', action='store_true',
                     help='feed raw uint8 [B,H,W,3] images (normalisation fused into the stem) instead of float32 [B,3,H,W]')
     ap.add_argument('--dump-ops', default=None, help='write the per-op timing table (profiling pass) to this JSON file')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write what the last timed step computed (annotations, sampled head outputs) as DIR/<name>.npy')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':

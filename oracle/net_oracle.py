@@ -13,8 +13,8 @@ path (paths relative to /root/reference/src/openpifpaf/):
 Attribute names and state_dict keys equal the reference's, so a reference
 `Shell` state_dict loads here unchanged; tests/test_network_lowering.py
 (test_oracle_net_equals_reference_modules, test_oracle_resnet_equals_reference_module) checks the
-two produce identical fields when /root/reference is importable (parity pinned
-against the Python reference imported in the build container).  It is the fp32
+two produce identical fields, against the reference modules' outputs stored by
+oracle/make_golden.py.  It is the fp32
 numerics reference for the CUDA kernels and the "port" CPU baseline of bench.py.
 """
 import torch

@@ -3,7 +3,8 @@
 Runs the UNMODIFIED reference (the staged package oracle/_ref_pkg, see build_ref.stage_package) on the bench
 workload: its own ``Shell`` built by its own ``network.Factory`` and its own ``Decoder.batch`` with the CPU C++
 ``CifCaf`` (decoder/decoder.py:114-137, decoder/cifcaf.py:224-277).  Used only by bench.py's reference legs
-(`--impl reference`, `cpu_baseline`, `library_baseline`) and by tests; the product never imports it.
+(`--impl reference`, `cpu_baseline`, `library_baseline`) and by tests; the product never imports it.  Where the package is not staged,
+the CPU legs run the port instead: oracle/net_oracle.py's Shell and the plain-C oracle decoder (`run_port_cpu`).
 
 Same workload as the CUDA arm:
   * same weights: the folded plan of openpifpaf_b200.network.random_plan (+ calibrated heads) is written into the
@@ -68,6 +69,20 @@ def shell_from_plan(openpifpaf, plan, base_name, workload='cocokp'):
     f.base_name, f.checkpoint = base_name, None
     openpifpaf.network.basenetworks.Resnet.pretrained = False
     shell, _ = f.factory(head_metas=head_metas(openpifpaf, workload))
+    return _load_plan(shell, plan)
+
+
+def port_shell_from_plan(plan, base_name, workload='cocokp'):
+    """oracle/net_oracle.py's restatement of the same Shell (same module and parameter names) carrying the weights
+    of a folded plan: the CPU arm's network when the reference package is not staged."""
+    from oracle import net_oracle
+    from openpifpaf_b200 import synth
+    shell = net_oracle.make_shell(base_name, n_keypoints=synth.WORKLOADS[workload][0],
+                                  n_connections=len(synth.skeleton_for(workload)), randomize_bn=False)
+    return _load_plan(shell, plan)
+
+
+def _load_plan(shell, plan):
     base = shell.base_net
     if plan['kind'] == 'shufflenetv2k':
         _set_conv_bn(base.input_block[0][0], base.input_block[0][1], (plan['input']['w'], plan['input']['b']))
@@ -151,9 +166,19 @@ def pick_threads(shell, size=321):
     return best
 
 
+def cpu_shell(plan, base_name, workload='cocokp'):
+    """The CPU arm's network: the reference's own Shell when the reference package is staged, else the port's."""
+    if available():
+        return shell_from_plan(import_reference(), plan, base_name, workload)
+    return port_shell_from_plan(plan, base_name, workload)
+
+
 def run_cpu(plan, base_name, workload, images, planted, steps, warmup, decoder_workers=0):
     """`steps` timed passes of Decoder.batch(model, images) on the host cores.  Returns a dict with the timing where
-    the reference measures it (decoder/decoder.py:116-118,129-132)."""
+    the reference measures it (decoder/decoder.py:116-118,129-132).  Without the staged reference package the same
+    step runs on the port (`run_port_cpu`); `kind` says which of the two ran."""
+    if not available():
+        return run_port_cpu(plan, base_name, workload, images, planted, steps, warmup)
     openpifpaf = import_reference()
     shell = shell_from_plan(openpifpaf, plan, base_name, workload)
     cores = pick_threads(shell)
@@ -176,7 +201,42 @@ def run_cpu(plan, base_name, workload, images, planted, steps, warmup, decoder_w
             n_ann = sum(len(r) for r in res)
         dt = time.perf_counter() - t0
     return {'seconds': dt, 'images': int(images.shape[0]) * steps, 'cores': cores, 'annotations_last_step': n_ann,
-            'nn_seconds': nn_t, 'decoder_seconds': dec_t, 'decoder_workers': int(decoder_workers)}
+            'nn_seconds': nn_t, 'decoder_seconds': dec_t, 'decoder_workers': int(decoder_workers), 'kind': 'reference'}
+
+
+def run_port_cpu(plan, base_name, workload, images, planted, steps, warmup):
+    """The step of `run_cpu` on the port: net_oracle's Shell forward on PyTorch-CPU fp32, then the plain-C oracle
+    (a bit-exact restatement of the reference's C++ CifCaf, tests/test_oracle.py) decoding the planted fields of
+    each image in turn."""
+    from oracle import cifcaf as oc
+    from openpifpaf_b200 import synth
+    shell = port_shell_from_plan(plan, base_name, workload)
+    cores = pick_threads(shell)
+    n_kp = synth.WORKLOADS[workload][0]
+    skeleton = np.asarray(synth.skeleton_for(workload), dtype=np.int64) - 1
+    stride = shell.base_net.stride
+    params = oc.default_params()
+
+    def step(batch):
+        t0 = time.perf_counter()
+        with torch.no_grad():
+            [h.cpu() for h in shell(batch)]
+        t1 = time.perf_counter()
+        anns = [oc.decode(planted['cif'][k], stride, planted['caf'][k], stride, skeleton, n_kp, params=params)[0]
+                for k in range(int(batch.shape[0]))]
+        return t1 - t0, time.perf_counter() - t1, sum(len(a) for a in anns)
+
+    for _ in range(warmup):
+        step(images[:1])
+    n_ann, nn_t, dec_t = 0, 0.0, 0.0
+    t0 = time.perf_counter()
+    for _ in range(steps):
+        dn, dd, n_ann = step(images)
+        nn_t += dn
+        dec_t += dd
+    dt = time.perf_counter() - t0
+    return {'seconds': dt, 'images': int(images.shape[0]) * steps, 'cores': cores, 'annotations_last_step': n_ann,
+            'nn_seconds': nn_t, 'decoder_seconds': dec_t, 'decoder_workers': 0, 'kind': 'port'}
 
 
 def run_library_gpu(plan, base_name, workload, images_dev, reps=3):

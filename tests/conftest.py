@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, 'tests')):
     if p not in sys.path:
@@ -11,13 +9,3 @@ for p in (ROOT, os.path.join(ROOT, 'tests')):
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run with -m gpu on the B200 box)')
-
-
-@pytest.fixture(scope='session')
-def have_reference():
-    """The compiled unmodified reference decoder (oracle/_ref) is loadable."""
-    from oracle import cifcaf as oc
-    if not oc.ref_available() and not os.path.isdir('/root/reference'):
-        pytest.skip('oracle/_ref not built and /root/reference absent')
-    oc.load_ref()
-    return oc

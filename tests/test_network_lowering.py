@@ -1,71 +1,37 @@
-"""CPU: (1) the oracle network equals the reference's own PyTorch modules (imported from /root/reference
-when present); (2) the product's host lowering (BN folding, physical channel placement, fused
+"""CPU: (1) the oracle network equals the reference's own PyTorch modules (their outputs stored by
+oracle/make_golden.py); (2) the product's host lowering (BN folding, physical channel placement, fused
 cat+channel_shuffle, head epilogue) reproduces the oracle network when its op list is interpreted on the CPU."""
-import importlib.util
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
 import torch
 
+import helpers
 import ops_emulator
 from openpifpaf_b200 import network
+from oracle import make_golden as mg
 from oracle import net_oracle
 
-REF_SRC = '/root/reference/src/openpifpaf'
+
+def reference_networks():
+    """the reference's own modules on oracle/make_golden.py's inputs (python -m oracle.make_golden reference)"""
+    return np.load(os.path.join(helpers.GOLDEN_DIR, 'reference_networks.npz'))
 
 
-def _load_reference_modules():
-    """Load basenetworks / heads / headmeta of the reference by path, without running the package
-    __init__ (which needs the compiled extension and optional dependencies)."""
-    top = types.ModuleType('refpifpaf')
-    top.__path__ = [REF_SRC]
-    sys.modules['refpifpaf'] = top
-    net_pkg = types.ModuleType('refpifpaf.network')
-    net_pkg.__path__ = [os.path.join(REF_SRC, 'network')]
-    sys.modules['refpifpaf.network'] = net_pkg
-
-    def load(name, path):
-        spec = importlib.util.spec_from_file_location(name, path)
-        mod = importlib.util.module_from_spec(spec)
-        sys.modules[name] = mod
-        spec.loader.exec_module(mod)
-        return mod
-
-    top.headmeta = load('refpifpaf.headmeta', os.path.join(REF_SRC, 'headmeta.py'))
-    base = load('refpifpaf.network.basenetworks', os.path.join(REF_SRC, 'network', 'basenetworks.py'))
-    heads = load('refpifpaf.network.heads', os.path.join(REF_SRC, 'network', 'heads.py'))
-    return top.headmeta, base, heads
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='/root/reference absent')
 def test_oracle_net_equals_reference_modules():
-    headmeta, base, heads = _load_reference_modules()
-    torch.manual_seed(0)
-    ref_base = base.ShuffleNetV2K('shufflenetv2k16', [4, 8, 4], [24, 348, 696, 1392, 1392])
-    kps = [str(i) for i in range(17)]
-    sk = [(1, 2)] * 19
-    cif = headmeta.Cif('cif', 'cocokp', keypoints=kps, sigmas=[0.1] * 17)
-    caf = headmeta.Caf('caf', 'cocokp', keypoints=kps, sigmas=[0.1] * 17, skeleton=sk)
-    ref_heads = [heads.CompositeField4(cif, 1392), heads.CompositeField4(caf, 1392)]
+    """net_oracle's shufflenetv2k16 + CompositeField4 heads == the reference's basenetworks.ShuffleNetV2K and
+    heads.CompositeField4 carrying the same (randomised) weights"""
+    g = reference_networks()
     oracle = net_oracle.make_shell('shufflenetv2k16', seed=3)
-    # same parameter names -> load the oracle's (randomised) weights into the reference modules
-    ref_base.load_state_dict(oracle.base_net.state_dict())
-    for rh, oh in zip(ref_heads, oracle.head_nets):
-        rh.load_state_dict(oh.state_dict())
-        rh.eval()
-    net_oracle.model_defaults(ref_base)
-    ref_base.eval()
-    x = torch.randn(1, 3, 97, 113)
+    x = mg.net_input('shufflenetv2k16')
+    assert mg.sha(x.numpy()) == str(g['shufflenetv2k16_input_sha256'])
     with torch.no_grad():
-        feat = ref_base(x)
-        want = [rh(feat) for rh in ref_heads]
         got = oracle(x)
-    for w, g in zip(want, got):
-        assert w.shape == g.shape
-        torch.testing.assert_close(g, w, rtol=0, atol=1e-5)
+    for name, gt in zip(('cif', 'caf'), got):
+        want = torch.from_numpy(g['shufflenetv2k16_' + name])
+        assert want.shape == gt.shape
+        torch.testing.assert_close(gt, want, rtol=0, atol=1e-5)
 
 
 @pytest.mark.parametrize('layout', ['bins', 'shuffle'])
@@ -230,21 +196,24 @@ def test_fused_and_unfused_lowerings_compute_the_same_network(fuse):
         assert float((g - wnt).abs().max()) < 2e-5 * max(1.0, float(wnt.abs().max()))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason='/root/reference absent')
 def test_oracle_resnet_equals_reference_module():
-    """SURVEY 8a row a3: the oracle Resnet wrapper == reference basenetworks.Resnet (max-pool removed, stride 16)."""
-    import torchvision
-    _, base, _ = _load_reference_modules()
-    base.Resnet.pretrained = False
-    ref = base.Resnet('resnet18', lambda pretrained: torchvision.models.resnet18(weights=None), 512)
-    assert ref.stride == 16
+    """SURVEY 8a row a3: the oracle Resnet wrapper == reference basenetworks.Resnet (max-pool removed, stride 16), on a
+    seeded sample of the output elements and on every channel's mean"""
+    g = reference_networks()
+    torch.manual_seed(0)
     oracle = net_oracle.make_base('resnet18')
-    ref.load_state_dict(oracle.state_dict())
-    ref.eval(); oracle.eval()
-    x = torch.randn(1, 3, 161, 161)
+    oracle.eval()
+    assert mg.sha(np.concatenate([p.detach().numpy().ravel() for p in oracle.parameters()])) == \
+        str(g['resnet18_weights_sha256'])
+    x = mg.net_input('resnet18')
+    assert mg.sha(x.numpy()) == str(g['resnet18_input_sha256'])
     with torch.no_grad():
-        torch.testing.assert_close(oracle(x), ref(x), rtol=0, atol=1e-5)
-    assert tuple(oracle(x).shape) == (1, 512, 11, 11)
+        out = oracle(x)
+    assert int(g['resnet18_stride']) == oracle.stride == 16
+    assert tuple(out.shape) == tuple(g['resnet18_shape']) == (1, 512, 11, 11)
+    torch.testing.assert_close(out.reshape(-1)[torch.from_numpy(mg.resnet_sample_index())],
+                               torch.from_numpy(g['resnet18_sample']), rtol=0, atol=1e-5)
+    torch.testing.assert_close(out[0].mean((1, 2)), torch.from_numpy(g['resnet18_channel_mean']), rtol=0, atol=1e-5)
 
 
 @pytest.mark.parametrize('name,shape', [('resnet18', (161, 161)), ('resnet50', (97, 113))])

@@ -1,6 +1,7 @@
-"""CPU: the plain-C oracle against the reference's outputs (golden vectors dumped from the
-unmodified reference build, and -- when oracle/_ref is present -- the reference itself, live)."""
+"""CPU: the plain-C oracle against the reference's outputs: golden vectors dumped from the unmodified reference
+build (oracle/make_golden.py), bit for bit at every stage."""
 import hashlib
+import os
 
 import numpy as np
 import pytest
@@ -8,10 +9,16 @@ import pytest
 import helpers
 from openpifpaf_b200 import synth
 from oracle import cifcaf as oc
+from oracle import make_golden as mg
 
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def reference_cases():
+    """the reference decoder's outputs on the cases below (python -m oracle.make_golden reference)"""
+    return np.load(os.path.join(helpers.GOLDEN_DIR, 'reference_oracle_cases.npz'))
 
 
 @pytest.mark.parametrize('path', helpers.golden_cases(), ids=lambda p: p.split('decoder_')[-1][:-4])
@@ -39,45 +46,38 @@ def test_golden_stored_fields_roundtrip():
     np.testing.assert_array_equal(ann, g['annotations'])
 
 
-@pytest.mark.parametrize('seed', range(4))
-def test_oracle_matches_live_reference(have_reference, seed):
-    ref = have_reference
-    f = synth.make_fields('cocokp', 21, 27, None, 100 + seed, n_distractors=4)
-    ref.ref_configure()
-    ra, ri, rt = ref.ref_decode(f['cif'], 16, f['caf'], 16, f['skeleton'], 17, taps=True)
+@pytest.mark.parametrize('seed', mg.LIVE_CIFCAF_SEEDS)
+def test_oracle_matches_live_reference(seed):
+    g = reference_cases()
+    f = mg.live_cifcaf_fields(seed)
+    assert synth.fields_digest(f['cif'], f['caf']) == str(g[f'cifcaf{seed}_fields_sha256'])
     oa, oi, ot = oc.decode(f['cif'], 16, f['caf'], 16, f['skeleton'], 17, taps=True)
-    np.testing.assert_array_equal(rt['cifhr'], ot['cifhr'])
-    np.testing.assert_array_equal(rt['seeds_vxys'], ot['seeds_vxys'])
-    for a, b in zip(rt['fwd'] + rt['bwd'], ot['fwd'] + ot['bwd']):
-        np.testing.assert_array_equal(a, b)
-    np.testing.assert_array_equal(ra, oa)
-    np.testing.assert_array_equal(ri, oi)
+    assert sha(ot['cifhr']) == str(g[f'cifcaf{seed}_cifhr_sha256'])
+    np.testing.assert_array_equal(ot['seeds_vxys'], g[f'cifcaf{seed}_seeds_vxys'])
+    for side in ('fwd', 'bwd'):
+        assert [len(x) for x in ot[side]] == list(g[f'cifcaf{seed}_n_{side}'])
+        assert sha(np.concatenate([x.reshape(-1, 7) for x in ot[side]])) == str(g[f'cifcaf{seed}_{side}_sha256'])
+    np.testing.assert_array_equal(oa, g[f'cifcaf{seed}_annotations'])
+    np.testing.assert_array_equal(oi, g[f'cifcaf{seed}_ids'])
 
 
-def test_oracle_initial_annotations_match_reference(have_reference):
-    ref = have_reference
-    f = synth.make_fields('cocokp', 41, 41, 3, 31)
-    ref.ref_configure()
-    base, _ = ref.ref_decode(f['cif'], 16, f['caf'], 16, f['skeleton'], 17)
-    init = base[:1].copy()
-    init[0, 5:] = 0.0          # keep a few joints of the first person, let the decoder regrow the rest
-    ids = np.array([42], dtype=np.int64)
-    ra, ri = ref.ref_decode(f['cif'], 16, f['caf'], 16, f['skeleton'], 17, initial_annotations=init, initial_ids=ids)
+def test_oracle_initial_annotations_match_reference():
+    g = reference_cases()
+    f = mg.initial_annotations_fields()
+    assert synth.fields_digest(f['cif'], f['caf']) == str(g['init_fields_sha256'])
+    init, ids = g['init_annotations'], g['init_ids']
     oa, oi = oc.decode(f['cif'], 16, f['caf'], 16, f['skeleton'], 17, initial_annotations=init, initial_ids=ids)
-    np.testing.assert_array_equal(ra, oa)
-    np.testing.assert_array_equal(ri, oi)
+    np.testing.assert_array_equal(oa, g['init_result_annotations'])
+    np.testing.assert_array_equal(oi, g['init_result_ids'])
     assert 42 in oi
 
 
-def test_oracle_grow_connection_blend_matches_reference(have_reference):
-    import torch
-    have_reference.load_ref()
-    rng = np.random.default_rng(0)
-    caf = rng.random((50, 7)).astype(np.float32) * np.array([1, 40, 40, 40, 40, 8, 8], dtype=np.float32)
+def test_oracle_grow_connection_blend_matches_reference():
+    g = reference_cases()
+    caf = mg.blend_caf()
     for only_max in (False, True):
-        want = torch.ops.openpifpaf_decoder.grow_connection_blend(torch.from_numpy(caf), 20.0, 20.0, 30.0, 1.0, only_max)
         got = oc.grow_connection_blend(caf, 20.0, 20.0, 30.0, 1.0, only_max)
-        assert list(want) == got
+        assert list(g[f'blend_only_max{int(only_max)}']) == got
 
 
 def test_empty_and_degenerate_fields():
@@ -103,13 +103,14 @@ def test_oracle_cifdet_matches_golden(path):
     assert len(cats) <= 120
 
 
-@pytest.mark.parametrize('seed', range(3))
-def test_oracle_cifdet_matches_live_reference(have_reference, seed):
-    f = synth.make_det_fields(80, 27, 21, 5 + 20 * seed, 200 + seed, n_distractors=6)
-    want = have_reference.ref_decode_det(f['field'], 16)
-    got = oc.decode_det(f['field'], 16)
-    for a, b in zip(want, got):
-        np.testing.assert_array_equal(a, b)
+@pytest.mark.parametrize('seed', mg.LIVE_CIFDET_SEEDS)
+def test_oracle_cifdet_matches_live_reference(seed):
+    g = reference_cases()
+    field = mg.live_cifdet_field(seed)
+    assert sha(field) == str(g[f'cifdet{seed}_field_sha256'])
+    got = oc.decode_det(field, 16)
+    for a, key in zip(got, ('categories', 'scores', 'boxes')):
+        np.testing.assert_array_equal(a, g[f'cifdet{seed}_{key}'])
     assert len(got[0]) >= 3
 
 

@@ -2,21 +2,18 @@
 
 CPU: the restatement of Pillow's ImagingResample (coefficient tables + integer arithmetic) against PIL.Image.resize
 itself -- Pillow is the third-party dependency the reference resizes with (transforms/scale.py:56-59); the meta dicts
-and the batched inverse_transform / json_data against the reference's own transforms / Annotation (when the staged
-reference package exists).  GPU: the kernels against PIL + torchvision's pad, and the whole raw-image path."""
+and the batched inverse_transform / json_data against the reference's own transforms / Annotation (their results
+stored by oracle/make_golden.py).  GPU: the kernels against PIL + torchvision's pad, and the whole raw-image path."""
+import json
 import os
-import subprocess
-import sys
-import textwrap
 
 import numpy as np
 import pytest
 import torch
 
+from helpers import GOLDEN_DIR
 from openpifpaf_b200 import preprocess as pp
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PKG = os.path.join(ROOT, 'oracle', '_ref_pkg')
+from oracle import make_golden as mg
 
 SIZES = [(480, 640, 641, 481), (375, 500, 321, 241), (100, 37, 161, 435), (600, 800, 400, 300), (33, 33, 33, 65),
          (720, 1280, 641, 360), (50, 50, 50, 50), (427, 640, 640, 427), (2, 3, 7, 5), (1080, 1920, 321, 180)]
@@ -58,57 +55,39 @@ def test_inverse_transform_and_json_batch_forms():
     assert len(js) == 5 and len(js[0]['keypoints']) == 51 and js[0]['score'] >= 0.001
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(PKG, 'openpifpaf', '_cpp.so')), reason='reference package not staged')
-def test_meta_and_annotations_equal_reference_transforms(tmp_path):
-    """the reference's own Predictor preprocessing (PIL path) and Annotation methods, run in a subprocess"""
-    script = textwrap.dedent('''
-        import sys, warnings
-        warnings.filterwarnings('ignore')
-        import numpy as np, PIL.Image, torch
-        import openpifpaf
-        from openpifpaf import transforms
-        import openpifpaf.transforms.scale as scale_mod
-        scale_mod.cv2 = None                         # the documented Pillow path (transforms/scale.py:56-59)
-        from openpifpaf_b200 import preprocess as pp
-        from openpifpaf.plugins.coco.constants import COCO_KEYPOINTS, COCO_PERSON_SKELETON, COCO_PERSON_SCORE_WEIGHTS
-        rng = np.random.default_rng(0)
-        for (h, w, long_edge, batched) in ((427, 640, 641, True), (480, 360, 321, True), (333, 500, 385, False), (200, 300, None, False)):
-            img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-            pre = [transforms.NormalizeAnnotations()]
-            if long_edge:
-                pre.append(transforms.RescaleAbsolute(long_edge, fast=True))
-            pre.append(transforms.CenterPad(long_edge) if batched else transforms.CenterPadTight(16))
-            torch.manual_seed(3)
-            image, anns, meta = transforms.Compose(pre)(PIL.Image.fromarray(img), [], None)
-            torch.manual_seed(3)
-            fill = int(torch.randint(0, 255, (1,)).item())
-            g = pp.GpuPreprocess.__new__(pp.GpuPreprocess)          # host logic only (no GPU here)
-            g.long_edge, g.batched, g.multiple = long_edge, batched, 16
-            (tw, th, ltrb, (cw, ch)), = g.plan([(w, h)])[0]
-            assert image.size == (cw, ch), (image.size, cw, ch)
-            canvas = np.empty((ch, cw, 3), dtype=np.uint8)
-            canvas[:] = (fill, fill, fill) if batched else pp.TIGHT_PAD_FILL
-            canvas[ltrb[1]:ltrb[1] + th, ltrb[0]:ltrb[0] + tw] = pp.resize_bilinear_reference(img, tw, th)
-            assert np.array_equal(np.asarray(image), canvas), 'resized + padded image differs'
-            mine = pp.reference_meta(w, h, tw, th, np.asarray(ltrb))
-            for k in ('offset', 'scale', 'valid_area', 'width_height'):
-                assert np.array_equal(np.asarray(meta[k], dtype=np.float64), np.asarray(mine[k], dtype=np.float64)), (k, meta[k], mine[k])
-            # annotations: inverse_transform + json_data
-            dec = rng.random((4, 17, 4)).astype(np.float32) * np.array([1, cw, ch, 9], dtype=np.float32)
-            dec[1, 5:11, 0] = 0.0
-            data, scales = pp.inverse_transform_batch(dec, mine)
-            js = pp.json_data_batch(data, scales, score_weights=COCO_PERSON_SCORE_WEIGHTS)
-            for i in range(4):
-                a = openpifpaf.Annotation(COCO_KEYPOINTS, COCO_PERSON_SKELETON, score_weights=COCO_PERSON_SCORE_WEIGHTS)
-                a.data[:, :2] = dec[i, :, 1:3]; a.data[:, 2] = dec[i, :, 0]; a.joint_scales[:] = dec[i, :, 3]
-                b = a.inverse_transform(meta)
-                assert np.array_equal(b.data, data[i]) and np.array_equal(b.joint_scales, scales[i])
-                assert b.json_data() == js[i], (b.json_data(), js[i])
-        print('PREPROCESS_REF_OK')
-    ''')
-    env = dict(os.environ, PYTHONPATH=f'{PKG}:{ROOT}')
-    r = subprocess.run([sys.executable, '-c', script], capture_output=True, text=True, env=env, cwd=str(tmp_path), timeout=600)
-    assert 'PREPROCESS_REF_OK' in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
+def test_meta_and_annotations_equal_reference_transforms():
+    """the reference's own Predictor preprocessing (PIL path) and Annotation methods, stored by oracle/make_golden.py"""
+    import hashlib
+    with open(os.path.join(GOLDEN_DIR, 'reference_transforms.json')) as f:
+        golden = json.load(f)
+    cases, score_weights = golden['cases'], golden['score_weights']
+    assert [(c['h'], c['w'], c['long_edge'], c['batched']) for c in cases] == list(mg.TRANSFORM_CASES)
+    rng = np.random.default_rng(0)
+    for (h, w, long_edge, batched), ref in zip(mg.TRANSFORM_CASES, cases):
+        img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+        torch.manual_seed(3)
+        fill = int(torch.randint(0, 255, (1,)).item())
+        g = pp.GpuPreprocess.__new__(pp.GpuPreprocess)          # host logic only (no GPU here)
+        g.long_edge, g.batched, g.multiple = long_edge, batched, 16
+        (tw, th, ltrb, (cw, ch)), = g.plan([(w, h)])[0]
+        assert ref['image_shape'] == [ch, cw, 3], (ref['image_shape'], cw, ch)
+        canvas = np.empty((ch, cw, 3), dtype=np.uint8)
+        canvas[:] = (fill, fill, fill) if batched else pp.TIGHT_PAD_FILL
+        canvas[ltrb[1]:ltrb[1] + th, ltrb[0]:ltrb[0] + tw] = pp.resize_bilinear_reference(img, tw, th)
+        assert hashlib.sha256(canvas.tobytes()).hexdigest() == ref['image_sha256'], 'resized + padded image differs'
+        mine = pp.reference_meta(w, h, tw, th, np.asarray(ltrb))
+        for k in ('offset', 'scale', 'valid_area', 'width_height'):
+            assert np.array_equal(np.asarray(ref['meta'][k], dtype=np.float64), np.asarray(mine[k], dtype=np.float64)), \
+                (k, ref['meta'][k], mine[k])
+        # annotations: inverse_transform + json_data
+        dec = rng.random((4, 17, 4)).astype(np.float32) * np.array([1, cw, ch, 9], dtype=np.float32)
+        dec[1, 5:11, 0] = 0.0
+        data, scales = pp.inverse_transform_batch(dec, mine)
+        js = pp.json_data_batch(data, scales, score_weights=score_weights)
+        for i, b in enumerate(ref['annotations']):
+            assert np.array_equal(np.asarray(b['data'], dtype=np.float32), data[i])
+            assert np.array_equal(np.asarray(b['joint_scales'], dtype=np.float32), scales[i])
+            assert b['json_data'] == js[i], (b['json_data'], js[i])
 
 
 @pytest.mark.gpu
