@@ -240,7 +240,12 @@ int pifpaf_image_fill_rgb(uint8_t* dst_dev, int64_t n_pixels, int32_t r, int32_t
  * modules (openpifpaf_b200/network.py) walks a Shell-like module, folds
  * BatchNorm (eval) into weights+bias and channel_shuffle/chunk into physical
  * channel placement, and emits these ops once; forward() replays them.
- * All weights are HOST f32 pointers (copied/converted at emit time).         */
+ * All weights are HOST f32 pointers (copied/converted at emit time).
+ *
+ * Activation codes: the `relu` / `dw_relu` argument of the ops below selects the activation fused into the epilogue,
+ * applied in f32 before the bf16 rounding (torchvision MobileNetV2 / V3 blocks, basenetworks.py:407-458):
+ *   0 none, 1 ReLU, 2 ReLU6 (torch.nn.ReLU6), 3 Hardswish (torch.nn.Hardswish: x * min(max(x + 3, 0), 6) / 6).
+ * Codes 2 and 3 need a 3x3 kernel in pifpaf_net_input_conv; pifpaf_net_dw_conv1x1_scatter accepts 0 and 1 only.                                                            */
 typedef struct pifpaf_net pifpaf_net_t;
 
 int pifpaf_net_create(pifpaf_net_t** out, int32_t device, int32_t max_batch);
@@ -291,10 +296,29 @@ int pifpaf_net_conv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, in
                     const float* bias, int32_t relu, int32_t out_tensor, int32_t out_col_off,
                     int32_t residual_tensor, int32_t residual_col_off);
 
-/* Depthwise kxk conv (basenetworks.py:228-231), weight [channels][k][k], + bias (folded BN) (+ReLU). */
+/* Depthwise kxk conv (basenetworks.py:228-231), weight [channels][k][k], + bias (folded BN) + activation code.
+ * Activation codes 2 and 3 need k = 3 or 5 and stride 1 or 2 (the MobileNet depthwise convs, torchvision
+ * InvertedResidual behind basenetworks.py:407-458); 3x3 convs of stride 1 or 2 and every depthwise conv followed
+ * by pifpaf_net_se_conv1x1 run on a kernel for any channel count (k_dwconv_nc). */
 int pifpaf_net_dwconv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, int32_t channels,
                       int32_t kernel, int32_t stride, int32_t pad, const float* weight, const float* bias,
                       int32_t relu, int32_t out_tensor, int32_t out_col_off);
+
+/* Squeeze-excitation + linear projection of a MobileNetV3 block (torchvision InvertedResidual with
+ * SqueezeExcitation, behind basenetworks.py:432-458): s = Hardsigmoid(fc2(ReLU(fc1(avgpool(x))))), then the 1x1
+ * projection conv + folded BN on x * s, no activation, optional residual add (use_res_connect; residual_tensor < 0:
+ * none).  in_tensor must be the whole output of the op emitted just before, a pifpaf_net_dwconv over `channels`
+ * channels with k = 3 or 5 and stride 1 or 2: that op then also writes per-tile channel sums of its f32 outputs
+ * (fixed-order reduction, no atomics: deterministic and independent of the batch).  Emits two ops: a squeeze-excitation
+ * kernel (one CTA per image: pooling, fc1, ReLU, fc2, Hardsigmoid) that writes per-image projection weights
+ * bf16(weight[n][k] * s[k]), and the projection as the implicit-GEMM conv with kernel 1, each 8 x 16 pixel tile
+ * reading the weights of its image.
+ * fc1_weight [squeeze][channels], fc1_bias [squeeze], fc2_weight [channels][squeeze], fc2_bias [channels];
+ * weight [n_out][channels], bias [n_out]. */
+int pifpaf_net_se_conv1x1(pifpaf_net_t* net, int32_t in_tensor, int32_t channels, int32_t squeeze,
+                          const float* fc1_weight, const float* fc1_bias, const float* fc2_weight, const float* fc2_bias,
+                          int32_t n_out, const float* weight, const float* bias, int32_t out_tensor,
+                          int32_t residual_tensor);
 
 /* Depthwise 5x5 (stride 1) -> BatchNorm -> 1x1 conv -> BatchNorm -> ReLU, the tail of InvertedResidualK.branch2
  * (basenetworks.py:219-226), as ONE kernel: the depthwise result is produced tile by tile straight into the
@@ -350,7 +374,8 @@ int pifpaf_net_forward_u8(pifpaf_net_t* net, const uint8_t* images_nhwc_dev, int
 
 /* Same as pifpaf_net_forward but brackets every op with CUDA events on `stream` and, after a final
  * synchronise, writes per-op milliseconds to op_ms[num_ops] (profiling leg of bench.py; never the
- * headline timing).  op_kind[i]: 0 input conv, 1 tcgen05 GEMM, 2 depthwise conv, 3 fused depthwise -> GEMM; op_flops/op_bytes are
+ * headline timing).  op_kind[i]: 0 input conv, 1 tcgen05 GEMM, 2 depthwise conv, 3 fused depthwise -> GEMM,
+ * 4 squeeze-excitation (pifpaf_net_se_conv1x1's first op); op_flops/op_bytes are
  * the algorithmic FLOPs and bytes (inputs + outputs + weights, each once) of op i for this batch. */
 int pifpaf_net_forward_timed(pifpaf_net_t* net, const float* images_dev, int32_t batch, int32_t gemm_impl,
                              void* stream, float* op_ms, int32_t* op_kind, double* op_flops, double* op_bytes);

@@ -84,6 +84,7 @@ SYMBOLS = {
     'pifpaf_net_conv': (ctypes.c_int, [VP, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, VP, VP, c_i32, c_i32, c_i32,
                                        c_i32, c_i32]),
     'pifpaf_net_dwconv': (ctypes.c_int, [VP, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, VP, VP, c_i32, c_i32, c_i32]),
+    'pifpaf_net_se_conv1x1': (ctypes.c_int, [VP, c_i32, c_i32, c_i32, VP, VP, VP, VP, c_i32, VP, VP, c_i32, c_i32]),
     'pifpaf_net_heads': (ctypes.c_int, [VP, c_i32, c_i32, c_i32, VP, VP, VP, VP, VP]),
     'pifpaf_net_heads_upsampled': (ctypes.c_int, [VP, c_i32, c_i32, c_i32, VP, VP, VP, c_i32, VP, VP]),
     'pifpaf_net_head_output': (ctypes.c_int, [VP, c_i32, P(VP), P(c_i32), P(c_i32), P(c_i32), P(c_i32)]),

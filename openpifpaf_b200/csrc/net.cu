@@ -217,7 +217,7 @@ struct GemmArgs {
     int M, N, K;                 // rows, real output channels, k extent (columns of the A view)
     int a_col0;                  // first column of the A view inside its tensor (TMA coordinate; multiple of 8)
     int block_n, n_blocks, m_blocks, num_k_blocks, stages;
-    int mode, relu;
+    int mode, relu;              // relu: activation code (act_f)
     const float* bias;           // [n_blocks * block_n], zero padded
     // plain / shuffle
     __nv_bfloat16* out; int ldo; int out_col_off;
@@ -247,6 +247,9 @@ struct GemmArgs {
     const __nv_bfloat16* res; int ld_res; int res_col_off;
     // debug (SIMT) operand views
     const __nv_bfloat16* a; int lda; const __nv_bfloat16* wgt; int ldw;
+    // per-image weights (implicit-GEMM conv only; squeeze-excitation projections): image b reads weight rows
+    // [b * w_img_rows, (b + 1) * w_img_rows) of B; 0 = one weight matrix for the whole batch
+    int w_img_rows;
 };
 
 constexpr int PH = 8, PW = 16;     // conv output patch per M tile (PH * PW == BM)
@@ -272,6 +275,13 @@ __device__ __forceinline__ float softplus_f(float x) {   // torch softplus beta=
     return x > 20.0f ? x : log1pf(expf(x));
 }
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.0f / (1.0f + expf(-x)); }
+// fused activation codes of the C ABI (include/pifpaf_b200.h): 0 none, 1 ReLU, 2 ReLU6, 3 Hardswish
+// (torch.nn.Hardswish: x * min(max(x + 3, 0), 6) / 6, here with the reciprocal: within one ulp); applied in f32 before
+// the bf16 rounding.  Codes 0..2 are one clamp whose bounds the compiler hoists out of the epilogue loops.
+__device__ __forceinline__ float act_f(float x, int act) {
+    if (act == 3) return x * fminf(fmaxf(x + 3.f, 0.f), 6.f) * (1.f / 6.f);
+    return fminf(fmaxf(x, act ? 0.f : -INFINITY), act == 2 ? 6.f : INFINITY);
+}
 
 // Blackwell 256-bit global store (STG.E.256): p must be 32-byte aligned
 __device__ __forceinline__ void st_global_256(void* p, uint32_t a, uint32_t b, uint32_t c, uint32_t d,
@@ -310,6 +320,9 @@ __device__ __forceinline__ void store_words(uint32_t* p, const uint32_t (&w)[CHU
 // by TMA) or nullptr to read it from global memory.
 // dest: the MODE_SCATTER destination table (shared memory in the tensor-core kernel: a global load per chunk put
 // 11 warps per issue on the long scoreboard, ncu round 1; global in the debug kernel)
+// EXT: activation codes 2 / 3 (act_f) and per-image weights; the EXT = false instantiations are the ReLU-only kernels
+// the ShuffleNetV2K / ResNet ops run (instruction for instruction the code they ran before activation codes existed)
+template <bool EXT>
 __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, int m, int n0, const float* acc,
                                                const float* bias, const __nv_bfloat16* src_row,
                                                const DestGroup* dest) {
@@ -350,7 +363,10 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, int m, int n0,
 #pragma unroll
         for (int j = 0; j < CHUNK; j += 2) {
             float a0 = acc[j] + bv[j], a1 = acc[j + 1] + bv[j + 1];
-            if (g.relu) { a0 = fmaxf(a0, 0.f); a1 = fmaxf(a1, 0.f); }
+            if (g.relu) {
+                if (EXT) { a0 = act_f(a0, g.relu); a1 = act_f(a1, g.relu); }
+                else { a0 = fmaxf(a0, 0.f); a1 = fmaxf(a1, 0.f); }
+            }
             w[j >> 1] = pack_bf16(a0, a1);
         }
         if (g.debug & 1) { if (w[0] == 0x12345u && w[5] == 0x54321u) g.dest[0].base[0] = __float2bfloat16(0.f); return; }
@@ -383,7 +399,10 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, int m, int n0,
 #pragma unroll
         for (int j = 0; j < CHUNK; j += 2) {
             float a0 = acc[j] + bv[j] + rv[j], a1 = acc[j + 1] + bv[j + 1] + rv[j + 1];
-            if (g.relu) { a0 = fmaxf(a0, 0.f); a1 = fmaxf(a1, 0.f); }
+            if (g.relu) {
+                if (EXT) { a0 = act_f(a0, g.relu); a1 = act_f(a1, g.relu); }
+                else { a0 = fmaxf(a0, 0.f); a1 = fmaxf(a1, 0.f); }
+            }
             w[j >> 1] = pack_bf16(a0, a1);
         }
         if (g.debug & 1) { if (w[0] == 0x12345u && w[5] == 0x54321u) g.out[0] = __float2bfloat16(0.f); return; }
@@ -407,7 +426,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, int m, int n0,
 #pragma unroll
     for (int j = 0; j < CHUNK; j++) {
         float a = acc[j] + bv[j];
-        if (g.relu) a = fmaxf(a, 0.f);
+        if (g.relu) a = EXT ? act_f(a, g.relu) : fmaxf(a, 0.f);
         const uint32_t src_bits = (j & 1) ? (sw[j >> 1] >> 16) : (sw[j >> 1] & 0xffffu);
         const __nv_bfloat16 hb = __float2bfloat16_rn(a);
         w[j] = src_bits | (static_cast<uint32_t>(__bfloat16_as_ushort(hb)) << 16);
@@ -424,6 +443,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmArgs& g, int m, int n0,
 }
 
 // ------------------------------------------------------------------ tcgen05 GEMM
+template <bool EXT>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 k_gemm_tc(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
           const __grid_constant__ CUtensorMap tmap_src, GemmArgs g) {
@@ -536,7 +556,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CU
                     } else {
                         tma_load_2d(sa, &tmap_a, &full_bar[stage], g.a_col0 + kb * BK, m_blk * BM);
                     }
-                    if (!g.b_resident) tma_load_2d(sb, &tmap_b, &full_bar[stage], kb * BK, n_blk * g.block_n);
+                    if (!g.b_resident) tma_load_2d(sb, &tmap_b, &full_bar[stage], kb * BK, n_blk * g.block_n + (EXT ? cimg * g.w_img_rows : 0));
                     if (++stage == g.stages) { stage = 0; phase ^= 1; }
                 }
                 if (g.src_tma) {
@@ -607,7 +627,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CU
                 for (int j = 0; j < CHUNK; j++) accf[j] = __uint_as_float(v[j]);
                 const int n0 = n_blk * g.block_n + c;
                 if (n0 < ((g.N + 7) & ~7))
-                    epilogue_chunk(g, m, n0, accf, bias_s + n0, g.src_tma ? src_tile_row + c : nullptr, dest_s);
+                    epilogue_chunk<EXT>(g, m, n0, accf, bias_s + n0, g.src_tma ? src_tile_row + c : nullptr, dest_s);
             };
             if (g.debug & 4) {                       // timing experiment: release the accumulator without reading it
                 for (int ci = c_begin; ci < c_end; ci++) {
@@ -688,6 +708,7 @@ __device__ __forceinline__ void mbar_arrive_leader(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PEER_BIT_MASK) : "memory");
 }
 
+template <bool EXT>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 k_gemm_tc2(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_bh, GemmArgs g) {
     extern __shared__ __align__(1024) unsigned char smem_raw2[];
@@ -828,7 +849,7 @@ k_gemm_tc2(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ C
 #pragma unroll
                 for (int j = 0; j < CHUNK; j++) accf[j] = __uint_as_float(v[j]);
                 const int n0 = n_blk * g.block_n + c;
-                if (n0 < ((g.N + 7) & ~7)) epilogue_chunk(g, m, n0, accf, bias_s + n0, nullptr, dest_s);
+                if (n0 < ((g.N + 7) & ~7)) epilogue_chunk<EXT>(g, m, n0, accf, bias_s + n0, nullptr, dest_s);
             };
             if (c_begin < c_end) tmem_ld16_async(t_row + (uint32_t)(c_begin * CHUNK), va);
             for (int ci = c_begin; ci < c_end; ci += 2) {
@@ -895,14 +916,14 @@ __global__ void __launch_bounds__(128) k_gemm_simt(GemmArgs g) {
                         for (int j = 0; j < CHUNK; j++) {
                             const int n = n0 + j;
                             const float wv = (n < g.N)
-                                ? __bfloat162float(g.wgt[(size_t)n * g.ldw + (size_t)tap * g.conv_cblocks * BK + k]) : 0.f;
+                                ? __bfloat162float(g.wgt[((size_t)b * g.w_img_rows + n) * g.ldw + (size_t)tap * g.conv_cblocks * BK + k]) : 0.f;
                             acc[j] = fmaf(a, wv, acc[j]);
                         }
                     }
                 }
             }
         }
-        if (n0 < ((g.N + 7) & ~7)) epilogue_chunk(g, m, n0, acc, g.bias + n0, nullptr, g.dest);
+        if (n0 < ((g.N + 7) & ~7)) epilogue_chunk<true>(g, m, n0, acc, g.bias + n0, nullptr, g.dest);
     }
 }
 
@@ -1515,6 +1536,162 @@ __global__ void __launch_bounds__(256) k_dwconv(DwArgs a) {
 }
 
 
+// Depthwise kxk (k = 3 or 5, stride 1 or 2) of the MobileNet blocks (torchvision InvertedResidual behind
+// basenetworks.py:407-458) with any fused activation code, on any channel count in 8-channel groups: the TMA kernels
+// above work on 64-channel items, which on the 16..72-channel tensors at 641^2 and 321^2 would spend most of their
+// shared memory and FMAs on fill.  One thread = 8 channels x DW_OX consecutive output pixels of one row, register
+// blocked like k_dwconv5.  Per image the items run channel group fastest, then the strip, then the row, so a warp
+// reads whole input rows.  CTA = (chunk of NIT * blockDim items, image); blockDim is a multiple of C8, so a thread
+// keeps its channel group over all its items.
+// Squeeze-excitation blocks (se_part != nullptr): the CTA also writes the sums of its f32 post-activation outputs per
+// channel to slot [image][chunk][channel], reduced in a fixed order without atomics -- deterministic, and independent
+// of the batch (the chunking depends on the image size only).  k_se reduces the slots.
+struct DwNcArgs { float* se_part; int nit, nslots; };
+
+template <int K, int S>
+__global__ void __launch_bounds__(256) k_dwconv_nc(DwArgs a, DwNcArgs x) {
+    constexpr int NCOL = (DW_OX - 1) * S + K;
+    const int b = blockIdx.y;
+    const int strips = (a.Wout + DW_OX - 1) / DW_OX;
+    const int per_img = a.Hout * strips * a.C8;
+    const int C = a.C8 * 8;
+    const int c8 = threadIdx.x % a.C8;
+    float sum[8];
+#pragma unroll
+    for (int j = 0; j < 8; j++) sum[j] = 0.f;
+    float bias[8];
+    {
+        const float4 b0 = __ldg(reinterpret_cast<const float4*>(a.bias + c8 * 8));
+        const float4 b1 = __ldg(reinterpret_cast<const float4*>(a.bias + c8 * 8 + 4));
+        bias[0] = b0.x; bias[1] = b0.y; bias[2] = b0.z; bias[3] = b0.w;
+        bias[4] = b1.x; bias[5] = b1.y; bias[6] = b1.z; bias[7] = b1.w;
+    }
+    const int t0 = blockIdx.x * blockDim.x * x.nit + threadIdx.x;
+    for (int it = 0; it < x.nit; it++) {
+        const int t = t0 + it * blockDim.x;
+        if (t >= per_img) break;
+        const int p = t / a.C8;
+        const int sx = p % strips, oy = p / strips;
+        const int ox0 = sx * DW_OX;
+        const int ix0 = ox0 * S - a.pad;
+        float acc[DW_OX][8];
+#pragma unroll
+        for (int o = 0; o < DW_OX; o++)
+#pragma unroll
+            for (int j = 0; j < 8; j++) acc[o][j] = bias[j];
+#pragma unroll
+        for (int ky = 0; ky < K; ky++) {
+            const int iy = oy * S - a.pad + ky;
+            if (iy < 0 || iy >= a.Hin) continue;
+            float w[K][8];
+#pragma unroll
+            for (int kx = 0; kx < K; kx++) {
+                const float* wp = a.weight + (size_t)(ky * K + kx) * C + c8 * 8;
+                const float4 w0 = __ldg(reinterpret_cast<const float4*>(wp));
+                const float4 w1 = __ldg(reinterpret_cast<const float4*>(wp + 4));
+                w[kx][0] = w0.x; w[kx][1] = w0.y; w[kx][2] = w0.z; w[kx][3] = w0.w;
+                w[kx][4] = w1.x; w[kx][5] = w1.y; w[kx][6] = w1.z; w[kx][7] = w1.w;
+            }
+            const __nv_bfloat16* rowp = a.in + ((size_t)(b * a.Hin + iy) * a.Win) * a.ld_in + a.in_col_off + c8 * 8;
+#pragma unroll
+            for (int col = 0; col < NCOL; col++) {
+                const int ix = ix0 + col;
+                if (ix < 0 || ix >= a.Win) continue;
+                const uint4 v = __ldg(reinterpret_cast<const uint4*>(rowp + (size_t)ix * a.ld_in));
+                float f[8];
+                unpack8(v, f);
+#pragma unroll
+                for (int o = 0; o < DW_OX; o++) {
+                    const int kx = col - o * S;       // compile-time after unrolling
+                    if (kx < 0 || kx >= K) continue;
+#pragma unroll
+                    for (int j = 0; j < 8; j++) acc[o][j] = fmaf(f[j], w[kx][j], acc[o][j]);
+                }
+            }
+        }
+#pragma unroll
+        for (int o = 0; o < DW_OX; o++) {
+            const int ox = ox0 + o;
+            if (ox >= a.Wout) continue;
+#pragma unroll
+            for (int j = 0; j < 8; j++) {
+                acc[o][j] = act_f(acc[o][j], a.relu);
+                sum[j] += acc[o][j];
+            }
+            uint4 ov;
+            ov.x = pack_bf16(acc[o][0], acc[o][1]); ov.y = pack_bf16(acc[o][2], acc[o][3]);
+            ov.z = pack_bf16(acc[o][4], acc[o][5]); ov.w = pack_bf16(acc[o][6], acc[o][7]);
+            *reinterpret_cast<uint4*>(a.out + ((size_t)(b * a.Hout + oy) * a.Wout + ox) * a.ld_out + a.out_col_off + c8 * 8) = ov;
+        }
+    }
+    if (x.se_part == nullptr) return;
+    __shared__ float s_sum[256][9];
+#pragma unroll
+    for (int j = 0; j < 8; j++) s_sum[threadIdx.x][j] = sum[j];
+    __syncthreads();
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        const int g = c >> 3, j = c & 7;
+        float v = 0.f;
+        for (int t = g; t < (int)blockDim.x; t += a.C8) v += s_sum[t][j];
+        x.se_part[((size_t)b * x.nslots + blockIdx.x) * C + c] = v;
+    }
+}
+
+// torchvision SqueezeExcitation (avg-pool -> fc1 -> ReLU -> fc2 -> Hardsigmoid -> x * s) folded into the weights of
+// the projection 1x1 that follows it: one CTA per image reduces the depthwise kernel's channel-sum slots in a fixed
+// order, runs the two small FCs and writes that image's projection weights bf16(W[n][k] * s[k]) in the B layout of
+// the implicit-GEMM conv (kernel 1), which then reads the rows of its image (GemmArgs::w_img_rows).
+struct SeArgs {
+    const float* part; int nslots, C8;      // [B][nslots][C8 * 8] channel sums (k_dwconv_nc)
+    float inv_hw;                           // 1 / (pixels of the depthwise output)
+    int channels, squeeze;
+    const float *w1, *b1, *w2, *b2;         // fc1 [squeeze][channels] + [squeeze], fc2 [channels][squeeze] + [channels]
+    const float* wproj;                     // f32 [n_pad][k_total] projection weights (folded BN), zero padded
+    int n_pad, k_total;
+    __nv_bfloat16* wimg;                    // [max_batch][n_pad][k_total]
+};
+
+constexpr int SE_THREADS = 512;
+
+__global__ void __launch_bounds__(SE_THREADS) k_se(SeArgs a) {
+    extern __shared__ float se_s[];         // pooled [C], hidden [squeeze], scale [C]
+    const int b = blockIdx.x, C = a.C8 * 8;
+    float* pooled = se_s;
+    float* hid = se_s + C;
+    float* sc = hid + a.squeeze;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        const float* p = a.part + (size_t)b * a.nslots * C + c;
+        float v = 0.f;
+        for (int i = 0; i < a.nslots; i++) v += p[(size_t)i * C];
+        pooled[c] = v * a.inv_hw;
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < a.squeeze; j += blockDim.x) {
+        float h = a.b1[j];
+        const float* w = a.w1 + (size_t)j * a.channels;
+        for (int c = 0; c < a.channels; c++) h = fmaf(w[c], pooled[c], h);
+        hid[j] = fmaxf(h, 0.f);
+    }
+    __syncthreads();
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        float s = 0.f;
+        if (c < a.channels) {
+            float v = a.b2[c];
+            const float* w = a.w2 + (size_t)c * a.squeeze;
+            for (int j = 0; j < a.squeeze; j++) v = fmaf(w[j], hid[j], v);
+            s = fminf(fmaxf(v + 3.f, 0.f), 6.f) / 6.f;      // torch.nn.Hardsigmoid
+        }
+        sc[c] = s;
+    }
+    __syncthreads();
+    const int n_w = a.n_pad * a.k_total;
+    __nv_bfloat16* out = a.wimg + (size_t)b * n_w;
+    for (int i = threadIdx.x; i < n_w; i += blockDim.x) {
+        const int k = i % a.k_total;
+        out[i] = __float2bfloat16_rn(a.wproj[i] * (k < C ? sc[k] : 0.f));
+    }
+}
+
 // ------------------------------------------------------------------ fused depthwise 5x5 -> 1x1 GEMM
 // InvertedResidualK branch2 tail (basenetworks.py:219-226: dw5x5, BN, 1x1, BN, ReLU) as ONE kernel: the depthwise
 // output never visits HBM.  Per CTA (persistent over 8 x 16 output-pixel patches == 128-row M tiles), per 64-channel
@@ -1753,7 +1930,7 @@ k_dw_gemm(const __grid_constant__ CUtensorMap tmap_win, const __grid_constant__ 
 #pragma unroll
                 for (int j = 0; j < CHUNK; j++) accf[j] = __uint_as_float(v[j]);
                 const int n0 = ci * CHUNK;
-                if (n0 < ((g.N + 7) & ~7)) epilogue_chunk(g, m, n0, accf, bias_s + n0, nullptr, dest_s);
+                if (n0 < ((g.N + 7) & ~7)) epilogue_chunk<false>(g, m, n0, accf, bias_s + n0, nullptr, dest_s);
             };
             tmem_ld16_async(t_row, va);
             for (int ci = 0; ci < n_chunks; ci += 2) {
@@ -1796,7 +1973,8 @@ struct InConvArgs {
     int B, Hin, Win, Hout, Wout, C8, kernel, stride, pad, relu;
 };
 
-template <int KS, bool U8>
+// EXT: activation codes 2 / 3 (the MobileNet stems); EXT = false is the ReLU-only kernel of the other backbones
+template <int KS, bool U8, bool EXT = false>
 __global__ void __launch_bounds__(256) k_input_conv(InConvArgs a) {
     // one thread = one output pixel, all output channels: the 3*k*k input samples are loaded once (registers for
     // k = 3, thread-local memory for k = 7) and reused for every 8-channel group; weights are broadcast reads
@@ -1879,7 +2057,7 @@ __global__ void __launch_bounds__(256) k_input_conv(InConvArgs a) {
             }
             if (a.relu) {
 #pragma unroll
-                for (int j = 0; j < 8; j++) acc[j] = fmaxf(acc[j], 0.f);
+                for (int j = 0; j < 8; j++) acc[j] = EXT ? act_f(acc[j], a.relu) : fmaxf(acc[j], 0.f);
             }
             uint4 o;
             o.x = pack_bf16(acc[0], acc[1]); o.y = pack_bf16(acc[2], acc[3]);
@@ -2054,7 +2232,7 @@ cudaError_t launch_k(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, 
 
 struct Tensor { int h, w, c; __nv_bfloat16* data; };
 
-enum OpKind { OP_INPUT_CONV, OP_GEMM, OP_DW, OP_FUSED };
+enum OpKind { OP_INPUT_CONV, OP_GEMM, OP_DW, OP_FUSED, OP_SE };
 
 struct Op {
     OpKind kind;
@@ -2068,6 +2246,8 @@ struct Op {
     DwArgs dw{};
     CUtensorMap tmap_dw{}; bool dw_tma = false;
     CUtensorMap tmap_dw_tc{}; bool dw_tc = false;      // tensor-core depthwise (k_dwconv5_tc)
+    DwNcArgs dwnc{}; bool dw_nc = false;               // k_dwconv_nc (MobileNet depthwise: k 3 / 5, any activation, SE sums)
+    SeArgs se{};                                       // OP_SE (k_se)
     // fused depthwise -> GEMM (OP_FUSED): g + tmap_dw (windows) + tmap_b
     FusedArgs fu{};
     // input conv
@@ -2302,6 +2482,86 @@ int emit_gemm(pifpaf_net* net, Op& op, int in_tensor, int in_col_off, int k_cols
     return rc;
 }
 
+// k_dwconv_nc work split: CTA = blockDim * nit items of one image, blockDim a multiple of C8 (so a thread keeps its
+// channel group); nit from the image size alone, so that the squeeze-excitation sum slots do not depend on the batch
+void plan_dw_nc(const DwArgs& a, DwNcArgs* x, int* block) {
+    const int bd = (256 / a.C8) * a.C8;
+    const int per_img = a.Hout * ((a.Wout + DW_OX - 1) / DW_OX) * a.C8;
+    x->nit = std::max(1, std::min(16, per_img / (bd * 16)));
+    x->nslots = (per_img + bd * x->nit - 1) / (bd * x->nit);
+    *block = bd;
+}
+
+// dense kxk conv as an implicit GEMM on tensor cores (8 x 16 output-pixel patches of one image per M tile).
+// wproj_f32 != nullptr: per-image weights (squeeze-excitation projection, kernel 1): B holds max_batch copies of the
+// weight matrix, written by k_se; *wproj_f32 receives the f32 weights [n_pad][k_total] k_se scales.
+int emit_conv_gemm(pifpaf_net* net, Op& op, int in_tensor, int in_col_off, int c_in, int kernel, int stride, int pad,
+                   int n_out, const float* weight, const float* bias, int relu, int out_tensor, int out_col_off,
+                   int residual_tensor, int residual_col_off, float** wproj_f32) {
+    const int nt = (int)net->tensors.size();
+    const Tensor& tin = net->tensors[in_tensor];
+    const Tensor& to = net->tensors[out_tensor];
+    const int ho = (tin.h + 2 * pad - kernel) / stride + 1, wo = (tin.w + 2 * pad - kernel) / stride + 1;
+    int block_n, n_blocks;
+    choose_block_n(n_out, &block_n, &n_blocks);
+    const int n_pad = block_n * n_blocks;
+    const int taps = kernel * kernel, cblocks = (c_in + BK - 1) / BK;
+    const int k_total = taps * cblocks * BK;
+    // torch weight [n_out][c_in][k][k] -> bf16 [n_pad][tap][cblocks*64]
+    std::vector<__nv_bfloat16> w((size_t)n_pad * k_total, __float2bfloat16(0.f));
+    for (int n = 0; n < n_out; n++)
+        for (int c = 0; c < c_in; c++)
+            for (int t = 0; t < taps; t++)
+                w[(size_t)n * k_total + (size_t)t * cblocks * BK + c] = __float2bfloat16(weight[((size_t)n * c_in + c) * taps + t]);
+    std::vector<float> b(n_pad, 0.f);
+    for (int n = 0; n < n_out; n++) b[n] = bias ? bias[n] : 0.f;
+    __nv_bfloat16* d_w = nullptr; float* d_b = nullptr;
+    int rc = net_upload(net, &d_b, b); if (rc != PIFPAF_OK) return rc;
+    uint64_t b_rows = (uint64_t)n_pad;
+    if (wproj_f32 == nullptr) {
+        rc = net_upload(net, &d_w, w); if (rc != PIFPAF_OK) return rc;
+    } else {
+        // per-image weights: k_se writes image b's copy of the weights into rows [b * n_pad, (b + 1) * n_pad)
+        PIFPAF_CHECK_ARG(kernel == 1, "per-image weights need kernel 1");
+        std::vector<float> wf(w.size(), 0.f);
+        for (int n = 0; n < n_out; n++)
+            for (int c = 0; c < c_in; c++) wf[(size_t)n * k_total + c] = weight[(size_t)n * c_in + c];
+        float* d_wf = nullptr;
+        rc = net_upload(net, &d_wf, wf); if (rc != PIFPAF_OK) return rc;
+        *wproj_f32 = d_wf;
+        b_rows = (uint64_t)net->max_batch * n_pad;
+        rc = net_alloc(net, &d_w, (size_t)b_rows * k_total, true); if (rc != PIFPAF_OK) return rc;
+        op.g.w_img_rows = n_pad;
+    }
+    GemmArgs& g = op.g;
+    g.N = n_out; g.K = c_in;
+    g.block_n = block_n; g.n_blocks = n_blocks;
+    g.num_k_blocks = taps * cblocks;
+    g.stages = choose_stages(block_n, n_blocks, g.num_k_blocks, false);
+    g.bias = d_b; g.mode = MODE_PLAIN; g.relu = relu;
+    g.out = to.data; g.ldo = to.c; g.out_col_off = out_col_off;
+    g.conv_k = kernel; g.conv_stride = stride; g.conv_pad = pad; g.conv_cblocks = cblocks;
+    g.Hi = tin.h; g.Wi = tin.w; g.Ho = ho; g.Wo = wo;
+    g.tiles_x = (wo + PW - 1) / PW; g.tiles_y = (ho + PH - 1) / PH;
+    g.a = tin.data + in_col_off; g.lda = tin.c; g.wgt = d_w; g.ldw = k_total;
+    if (residual_tensor >= 0) {
+        PIFPAF_CHECK_ARG(residual_tensor < nt, "bad residual tensor");
+        const Tensor& tr = net->tensors[residual_tensor];
+        PIFPAF_CHECK_ARG(tr.h == ho && tr.w == wo && residual_col_off % 8 == 0 && residual_col_off + n_out <= tr.c,
+                         "residual tensor shape mismatch");
+        g.res = tr.data; g.ld_res = tr.c; g.res_col_off = residual_col_off;
+    }
+    op.a_tensor = in_tensor; op.rows_per_image = ho * wo; op.tiles_per_image = g.tiles_x * g.tiles_y;
+    op.smem = gemm_smem_bytes(block_n, n_blocks, g.stages, false);
+    op.flops_per_image = 2.0 * (double)ho * wo * n_out * c_in * taps;
+    op.bytes_per_image = (double)tin.h * tin.w * c_in * 2.0 + (double)ho * wo * n_out * 2.0 * (residual_tensor >= 0 ? 2.0 : 1.0);
+    op.weight_bytes = (double)n_out * c_in * taps * 2.0;
+    rc = make_tmap_conv(&op.tmap_a, tin.data + in_col_off, (uint64_t)c_in, (uint64_t)tin.w, (uint64_t)tin.h,
+                        (uint64_t)net->max_batch, (uint64_t)tin.c, stride);
+    if (rc != PIFPAF_OK) return rc;
+    return make_tmap(&op.tmap_b, d_w, b_rows, (uint64_t)k_total, (uint64_t)k_total, (uint32_t)block_n);
+}
+
 }  // namespace
 
 extern "C" {
@@ -2328,13 +2588,15 @@ int pifpaf_net_create(pifpaf_net_t** out, int32_t device, int32_t max_batch) {
     if (const char* e = std::getenv("PIFPAF_GEMM_MC")) net->gemm_mc = std::atoi(e);
     if (const char* e = std::getenv("PIFPAF_GEMM_DEBUG")) net->gemm_debug = std::atoi(e);
     if (const char* e = std::getenv("PIFPAF_GEMM_PAIR")) net->gemm_pair = std::atoi(e);
-    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc2, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
     if (const char* e = std::getenv("PIFPAF_DW_TC")) net->dw_tc = std::atoi(e);
     if (const char* e = std::getenv("PIFPAF_DW_TC_PWID")) net->dw_tc_pwid = std::atoi(e) == 16 ? 16 : 12;
     if (const char* e = std::getenv("PIFPAF_DW_TC_BO")) net->dw_tc_bo = std::atoi(e) != 0;
     PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_dwconv5_tc<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
     PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_dwconv5_tc<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+    PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_gemm_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
     PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_dwconv5_tma<1, DW1_TH, DW1_TW, 4, 3>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, DwS1::SMEM));
     PIFPAF_CUDA_TRY(cudaFuncSetAttribute(k_dwconv5_tma<2, DW2_TH, DW2_TW, 4, 2>,
@@ -2370,11 +2632,13 @@ int pifpaf_net_input_conv(pifpaf_net_t* net, int32_t in_h, int32_t in_w, int32_t
                           int32_t pad, int32_t c_out, const float* weight, const float* bias,
                           int32_t relu, int32_t out_tensor) {
     PIFPAF_CHECK_ARG(net != nullptr && weight != nullptr, "null argument");
+    PIFPAF_CHECK_ARG(relu >= 0 && relu <= 3, "activation code must be 0..3");
     PIFPAF_CHECK_ARG(out_tensor >= 0 && out_tensor < (int)net->tensors.size(), "bad tensor id");
     const Tensor& to = net->tensors[out_tensor];
     const int ho = (in_h + 2 * pad - kernel) / stride + 1, wo = (in_w + 2 * pad - kernel) / stride + 1;
     PIFPAF_CHECK_ARG(to.h == ho && to.w == wo && to.c >= pad8(c_out), "output tensor shape mismatch");
     PIFPAF_CHECK_ARG(kernel == 1 || kernel == 3 || kernel == 5 || kernel == 7, "input conv kernel must be 1, 3, 5 or 7");
+    PIFPAF_CHECK_ARG(relu <= 1 || kernel == 3, "activation codes 2 and 3 need a 3x3 input conv");
     PIFPAF_CUDA_TRY(cudaSetDevice(net->device));
     const int C = pad8(c_out);
     std::vector<float> w((size_t)3 * kernel * kernel * C, 0.f), b(C, 0.f);
@@ -2406,6 +2670,7 @@ int pifpaf_net_conv1x1(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off,
                        int32_t out_tensor, int32_t out_col_off,
                        int32_t shuffle_src_tensor, int32_t shuffle_src_col_off) {
     PIFPAF_CHECK_ARG(net != nullptr && weight != nullptr, "null argument");
+    PIFPAF_CHECK_ARG(relu >= 0 && relu <= 3, "activation code must be 0..3");
     const int nt = (int)net->tensors.size();
     PIFPAF_CHECK_ARG(in_tensor >= 0 && in_tensor < nt && out_tensor >= 0 && out_tensor < nt, "bad tensor id");
     PIFPAF_CHECK_ARG(k_cols >= 1 && n_out >= 1, "bad conv size");
@@ -2455,6 +2720,7 @@ int pifpaf_net_conv1x1_scatter(pifpaf_net_t* net, int32_t in_tensor, int32_t in_
                                const int32_t* piece_tensor, const int32_t* piece_tensor_col) {
     PIFPAF_CHECK_ARG(net != nullptr && weight != nullptr && piece_col0 && piece_count && piece_tensor && piece_tensor_col,
                      "null argument");
+    PIFPAF_CHECK_ARG(relu >= 0 && relu <= 3, "activation code must be 0..3");
     const int nt = (int)net->tensors.size();
     PIFPAF_CHECK_ARG(in_tensor >= 0 && in_tensor < nt, "bad tensor id");
     PIFPAF_CHECK_ARG(k_cols >= 1 && n_out >= 16 && n_out % 16 == 0 && n_pieces >= 1, "bad conv size");
@@ -2497,6 +2763,7 @@ int pifpaf_net_conv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, in
                     const float* bias, int32_t relu, int32_t out_tensor, int32_t out_col_off,
                     int32_t residual_tensor, int32_t residual_col_off) {
     PIFPAF_CHECK_ARG(net != nullptr && weight != nullptr, "null argument");
+    PIFPAF_CHECK_ARG(relu >= 0 && relu <= 3, "activation code must be 0..3");
     const int nt = (int)net->tensors.size();
     PIFPAF_CHECK_ARG(in_tensor >= 0 && in_tensor < nt && out_tensor >= 0 && out_tensor < nt, "bad tensor id");
     PIFPAF_CHECK_ARG(kernel >= 1 && kernel <= 7 && stride >= 1 && stride <= 2 && pad >= 0, "unsupported conv geometry");
@@ -2530,49 +2797,8 @@ int pifpaf_net_conv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, in
         return PIFPAF_OK;
     }
     Op op; op.kind = OP_GEMM;
-    int block_n, n_blocks;
-    choose_block_n(n_out, &block_n, &n_blocks);
-    const int n_pad = block_n * n_blocks;
-    const int taps = kernel * kernel, cblocks = (c_in + BK - 1) / BK;
-    const int k_total = taps * cblocks * BK;
-    // torch weight [n_out][c_in][k][k] -> bf16 [n_pad][tap][cblocks*64]
-    std::vector<__nv_bfloat16> w((size_t)n_pad * k_total, __float2bfloat16(0.f));
-    for (int n = 0; n < n_out; n++)
-        for (int c = 0; c < c_in; c++)
-            for (int t = 0; t < taps; t++)
-                w[(size_t)n * k_total + (size_t)t * cblocks * BK + c] = __float2bfloat16(weight[((size_t)n * c_in + c) * taps + t]);
-    std::vector<float> b(n_pad, 0.f);
-    for (int n = 0; n < n_out; n++) b[n] = bias ? bias[n] : 0.f;
-    __nv_bfloat16* d_w = nullptr; float* d_b = nullptr;
-    int rc = net_upload(net, &d_w, w); if (rc != PIFPAF_OK) return rc;
-    rc = net_upload(net, &d_b, b); if (rc != PIFPAF_OK) return rc;
-    GemmArgs& g = op.g;
-    g.N = n_out; g.K = c_in;
-    g.block_n = block_n; g.n_blocks = n_blocks;
-    g.num_k_blocks = taps * cblocks;
-    g.stages = choose_stages(block_n, n_blocks, g.num_k_blocks, false);
-    g.bias = d_b; g.mode = MODE_PLAIN; g.relu = relu;
-    g.out = to.data; g.ldo = to.c; g.out_col_off = out_col_off;
-    g.conv_k = kernel; g.conv_stride = stride; g.conv_pad = pad; g.conv_cblocks = cblocks;
-    g.Hi = tin.h; g.Wi = tin.w; g.Ho = ho; g.Wo = wo;
-    g.tiles_x = (wo + PW - 1) / PW; g.tiles_y = (ho + PH - 1) / PH;
-    g.a = tin.data + in_col_off; g.lda = tin.c; g.wgt = d_w; g.ldw = k_total;
-    if (residual_tensor >= 0) {
-        PIFPAF_CHECK_ARG(residual_tensor < nt, "bad residual tensor");
-        const Tensor& tr = net->tensors[residual_tensor];
-        PIFPAF_CHECK_ARG(tr.h == ho && tr.w == wo && residual_col_off % 8 == 0 && residual_col_off + n_out <= tr.c,
-                         "residual tensor shape mismatch");
-        g.res = tr.data; g.ld_res = tr.c; g.res_col_off = residual_col_off;
-    }
-    op.a_tensor = in_tensor; op.rows_per_image = ho * wo; op.tiles_per_image = g.tiles_x * g.tiles_y;
-    op.smem = gemm_smem_bytes(block_n, n_blocks, g.stages, false);
-    op.flops_per_image = 2.0 * (double)ho * wo * n_out * c_in * taps;
-    op.bytes_per_image = (double)tin.h * tin.w * c_in * 2.0 + (double)ho * wo * n_out * 2.0 * (residual_tensor >= 0 ? 2.0 : 1.0);
-    op.weight_bytes = (double)n_out * c_in * taps * 2.0;
-    rc = make_tmap_conv(&op.tmap_a, tin.data + in_col_off, (uint64_t)c_in, (uint64_t)tin.w, (uint64_t)tin.h,
-                        (uint64_t)net->max_batch, (uint64_t)tin.c, stride);
-    if (rc != PIFPAF_OK) return rc;
-    rc = make_tmap(&op.tmap_b, d_w, (uint64_t)n_pad, (uint64_t)k_total, (uint64_t)k_total, (uint32_t)block_n);
+    int rc = emit_conv_gemm(net, op, in_tensor, in_col_off, c_in, kernel, stride, pad, n_out, weight, bias, relu,
+                            out_tensor, out_col_off, residual_tensor, residual_col_off, nullptr);
     if (rc != PIFPAF_OK) return rc;
     net->ops.push_back(op);
     return PIFPAF_OK;
@@ -2609,7 +2835,15 @@ int pifpaf_net_dwconv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, 
     a.kernel = kernel; a.stride = stride; a.pad = pad; a.relu = relu;
     op.flops_per_image = 2.0 * ho * wo * channels * (double)kernel * kernel;
     op.bytes_per_image = ((double)tin.h * tin.w + (double)ho * wo) * channels * 2.0;
-    if (kernel == 5 && (stride == 1 || stride == 2)) {
+    const bool nc_geometry = (kernel == 3 || kernel == 5) && (stride == 1 || stride == 2);
+    PIFPAF_CHECK_ARG(relu >= 0 && relu <= 3, "activation code must be 0..3");
+    PIFPAF_CHECK_ARG(relu <= 1 || nc_geometry, "activation codes 2 and 3 need a 3x3 or 5x5 depthwise conv of stride 1 or 2");
+    if (nc_geometry && (kernel == 3 || relu >= 2)) {
+        // MobileNet depthwise convs: k_dwconv_nc (5x5 with ReLU or none stays on the TMA kernels below unless a
+        // squeeze-excitation follows, pifpaf_net_se_conv1x1)
+        PIFPAF_CHECK_ARG(C / 8 <= 256, "depthwise conv of more than 2048 channels");
+        op.dw_nc = true;
+    } else if (kernel == 5 && (stride == 1 || stride == 2)) {
         const uint32_t bw = stride == 1 ? DwS1::IW : DwS2::IW;
         const uint32_t bh = stride == 1 ? DwS1::IH : DwS2::IH;
         rc = make_tmap_dw(&op.tmap_dw, tin.data + in_col_off, (uint64_t)C, (uint64_t)tin.w, (uint64_t)tin.h,
@@ -2626,6 +2860,64 @@ int pifpaf_net_dwconv(pifpaf_net_t* net, int32_t in_tensor, int32_t in_col_off, 
         }
     }
     net->ops.push_back(op);
+    return PIFPAF_OK;
+}
+
+int pifpaf_net_se_conv1x1(pifpaf_net_t* net, int32_t in_tensor, int32_t channels, int32_t squeeze,
+                          const float* fc1_weight, const float* fc1_bias, const float* fc2_weight, const float* fc2_bias,
+                          int32_t n_out, const float* weight, const float* bias, int32_t out_tensor,
+                          int32_t residual_tensor) {
+    PIFPAF_CHECK_ARG(net != nullptr && fc1_weight && fc1_bias && fc2_weight && fc2_bias && weight, "null argument");
+    const int nt = (int)net->tensors.size();
+    PIFPAF_CHECK_ARG(in_tensor >= 0 && in_tensor < nt && out_tensor >= 0 && out_tensor < nt && residual_tensor < nt,
+                     "bad tensor id");
+    PIFPAF_CHECK_ARG(channels >= 1 && channels <= 2048 && squeeze >= 1 && squeeze <= 2048 && n_out >= 1, "bad SE size");
+    const Tensor& tin = net->tensors[in_tensor];
+    const Tensor& to = net->tensors[out_tensor];
+    PIFPAF_CHECK_ARG(tin.h == to.h && tin.w == to.w, "the projection keeps the spatial shape");
+    PIFPAF_CHECK_ARG(!net->ops.empty() && net->ops.back().kind == OP_DW, "squeeze-excitation must follow a depthwise conv");
+    {
+        const DwArgs& d = net->ops.back().dw;
+        PIFPAF_CHECK_ARG(d.out == tin.data && d.out_col_off == 0 && d.C8 * 8 == pad8(channels),
+                         "squeeze-excitation input must be the whole output of the preceding depthwise conv");
+        PIFPAF_CHECK_ARG((d.kernel == 3 || d.kernel == 5) && (d.stride == 1 || d.stride == 2),
+                         "squeeze-excitation needs a 3x3 or 5x5 depthwise conv of stride 1 or 2");
+    }
+    PIFPAF_CUDA_TRY(cudaSetDevice(net->device));
+    DwNcArgs nc{}; int block = 0;
+    plan_dw_nc(net->ops.back().dw, &nc, &block);
+    const int C = pad8(channels);
+    float* d_part = nullptr;
+    int rc = net_alloc(net, &d_part, (size_t)net->max_batch * nc.nslots * C, true); if (rc != PIFPAF_OK) return rc;
+    nc.se_part = d_part;
+    {
+        Op& dw = net->ops.back();
+        dw.dw_nc = true;
+        dw.dwnc = nc;
+        dw.bytes_per_image += (double)nc.nslots * C * 4.0;
+    }
+    Op gop; gop.kind = OP_GEMM;
+    float* d_wproj = nullptr;
+    rc = emit_conv_gemm(net, gop, in_tensor, 0, channels, 1, 1, 0, n_out, weight, bias, 0, out_tensor, 0,
+                        residual_tensor, 0, &d_wproj);
+    if (rc != PIFPAF_OK) return rc;
+    Op op; op.kind = OP_SE;
+    float *d_w1 = nullptr, *d_b1 = nullptr, *d_w2 = nullptr, *d_b2 = nullptr;
+    rc = net_upload(net, &d_w1, std::vector<float>(fc1_weight, fc1_weight + (size_t)squeeze * channels)); if (rc != PIFPAF_OK) return rc;
+    rc = net_upload(net, &d_b1, std::vector<float>(fc1_bias, fc1_bias + squeeze)); if (rc != PIFPAF_OK) return rc;
+    rc = net_upload(net, &d_w2, std::vector<float>(fc2_weight, fc2_weight + (size_t)channels * squeeze)); if (rc != PIFPAF_OK) return rc;
+    rc = net_upload(net, &d_b2, std::vector<float>(fc2_bias, fc2_bias + channels)); if (rc != PIFPAF_OK) return rc;
+    SeArgs& a = op.se;
+    a.part = d_part; a.nslots = nc.nslots; a.C8 = C / 8; a.inv_hw = 1.0f / (float)(tin.h * tin.w);
+    a.channels = channels; a.squeeze = squeeze;
+    a.w1 = d_w1; a.b1 = d_b1; a.w2 = d_w2; a.b2 = d_b2;
+    a.wproj = d_wproj; a.n_pad = gop.g.block_n * gop.g.n_blocks; a.k_total = gop.g.ldw;
+    a.wimg = const_cast<__nv_bfloat16*>(gop.g.wgt);
+    op.flops_per_image = 4.0 * channels * squeeze + (double)a.n_pad * a.k_total;
+    op.bytes_per_image = (double)nc.nslots * C * 4.0 + (double)a.n_pad * a.k_total * 2.0;
+    op.weight_bytes = (2.0 * channels * squeeze + channels + squeeze) * 4.0 + (double)a.n_pad * a.k_total * 4.0;
+    net->ops.push_back(op);
+    net->ops.push_back(gop);
     return PIFPAF_OK;
 }
 
@@ -2833,11 +3125,13 @@ static int net_forward_impl(pifpaf_net_t* net, const float* images_dev, int32_t 
             if (u8 != nullptr) {
                 a.in_u8 = u8->images;
                 for (int c = 0; c < 3; c++) { a.mean[c] = u8->mean[c]; a.stdev[c] = u8->stdev[c]; }
-                if (a.kernel == 3) k_input_conv<3, true><<<grid, 256, smem, st>>>(a);
+                if (a.relu >= 2) k_input_conv<3, true, true><<<grid, 256, smem, st>>>(a);
+                else if (a.kernel == 3) k_input_conv<3, true><<<grid, 256, smem, st>>>(a);
                 else if (a.kernel == 7) k_input_conv<7, true><<<grid, 256, smem, st>>>(a);
                 else if (a.kernel == 5) k_input_conv<5, true><<<grid, 256, smem, st>>>(a);
                 else k_input_conv<1, true><<<grid, 256, smem, st>>>(a);
-            } else if (a.kernel == 3) k_input_conv<3, false><<<grid, 256, smem, st>>>(a);
+            } else if (a.relu >= 2) k_input_conv<3, false, true><<<grid, 256, smem, st>>>(a);
+            else if (a.kernel == 3) k_input_conv<3, false><<<grid, 256, smem, st>>>(a);
             else if (a.kernel == 7) k_input_conv<7, false><<<grid, 256, smem, st>>>(a);
             else if (a.kernel == 5) k_input_conv<5, false><<<grid, 256, smem, st>>>(a);
             else k_input_conv<1, false><<<grid, 256, smem, st>>>(a);
@@ -2850,10 +3144,23 @@ static int net_forward_impl(pifpaf_net_t* net, const float* images_dev, int32_t 
             const int grid = std::min(g.m_blocks, n_sm);
             PIFPAF_CUDA_TRY(launch_k(pdl, k_dw_gemm<1>, dim3(grid), dim3(FD_THREADS), op.smem, st, op.tmap_dw, op.tmap_b, g, op.fu));
             PIFPAF_LAUNCH_CHECK();
+        } else if (op.kind == OP_SE) {
+            const size_t smem = sizeof(float) * (2 * (size_t)op.se.C8 * 8 + op.se.squeeze);
+            k_se<<<batch, SE_THREADS, smem, st>>>(op.se);
+            PIFPAF_LAUNCH_CHECK();
         } else if (op.kind == OP_DW) {
             DwArgs a = op.dw;
             a.B = batch;
-            if (op.dw_tc && gemm_impl == 0) {
+            if (op.dw_nc) {
+                DwNcArgs x = op.dwnc; int block = 0;
+                plan_dw_nc(a, &x, &block);
+                x.se_part = op.dwnc.se_part;
+                const dim3 grid((unsigned)x.nslots, (unsigned)batch);
+                if (a.kernel == 3 && a.stride == 1) k_dwconv_nc<3, 1><<<grid, block, 0, st>>>(a, x);
+                else if (a.kernel == 3) k_dwconv_nc<3, 2><<<grid, block, 0, st>>>(a, x);
+                else if (a.stride == 1) k_dwconv_nc<5, 1><<<grid, block, 0, st>>>(a, x);
+                else k_dwconv_nc<5, 2><<<grid, block, 0, st>>>(a, x);
+            } else if (op.dw_tc && gemm_impl == 0) {
                 const int cblks = (a.C8 + 7) / 8;
                 const long long total = (long long)batch * ((a.Hout + DT_TH - 1) / DT_TH) * ((a.Wout + DT_TW - 1) / DT_TW) * cblks;
                 const int grid = (int)std::min<long long>(total, (long long)n_sm);
@@ -2907,6 +3214,7 @@ static int net_forward_impl(pifpaf_net_t* net, const float* images_dev, int32_t 
                 for (int i = 0; i < net->n_heads; i++) g.head_base[i] = net->head_out[net->head_cur][i];
             g.M = batch * op.rows_per_image;
             g.m_blocks = g.conv_k > 0 ? batch * op.tiles_per_image : (g.M + BM - 1) / BM;
+            const bool ext = g.relu >= 2 || g.w_img_rows > 0;
             if (gemm_impl == 1) {
                 const long long jobs = (long long)g.m_blocks * 4 * (g.n_blocks * g.block_n / CHUNK);
                 const int grid = (int)std::min<long long>((jobs + 3) / 4, (long long)n_sm * 16);
@@ -2917,14 +3225,14 @@ static int net_forward_impl(pifpaf_net_t* net, const float* images_dev, int32_t 
                 const int max_pairs = std::max(1, n_sm / 2);
                 int pairs = std::min(max_pairs, m2 * g.n_blocks);
                 if (g.b_resident) pairs = std::max(1, std::min(max_pairs / g.n_blocks, m2)) * g.n_blocks;
-                PIFPAF_CUDA_TRY(launch_kc(pdl, 2, k_gemm_tc2, dim3(2 * pairs), dim3(GEMM_THREADS), op.pair_smem, st, op.tmap_a,
+                PIFPAF_CUDA_TRY(launch_kc(pdl, 2, ext ? k_gemm_tc2<true> : k_gemm_tc2<false>, dim3(2 * pairs), dim3(GEMM_THREADS), op.pair_smem, st, op.tmap_a,
                                           op.tmap_bh, g));
             } else {
                 const int tiles = g.m_blocks * g.n_blocks;
                 int grid = std::min(tiles, n_sm);
                 if (g.b_resident) grid = std::max(1, std::min(n_sm / g.n_blocks, g.m_blocks)) * g.n_blocks;
                 // multicast pairs need at least one whole cluster and whole clusters only (grid is a multiple of n_blocks == 2)
-                PIFPAF_CUDA_TRY(launch_kc(pdl, g.mc ? 2 : 1, k_gemm_tc, dim3(grid), dim3(GEMM_THREADS), op.smem, st, op.tmap_a,
+                PIFPAF_CUDA_TRY(launch_kc(pdl, g.mc ? 2 : 1, ext ? k_gemm_tc<true> : k_gemm_tc<false>, dim3(grid), dim3(GEMM_THREADS), op.smem, st, op.tmap_a,
                                           op.tmap_b, (g.src_tma || g.mc) ? op.tmap_src : op.tmap_a, g));
             }
             PIFPAF_LAUNCH_CHECK();
@@ -2967,7 +3275,7 @@ int pifpaf_net_forward_timed(pifpaf_net_t* net, const float* images_dev, int32_t
     for (size_t i = 0; i < n && rc == PIFPAF_OK; i++) {
         cudaEventElapsedTime(&op_ms[i], ev[i], ev[i + 1]);
         const Op& op = net->ops[i];
-        if (op_kind) op_kind[i] = op.kind == OP_INPUT_CONV ? 0 : (op.kind == OP_GEMM ? 1 : (op.kind == OP_DW ? 2 : 3));
+        if (op_kind) op_kind[i] = op.kind == OP_INPUT_CONV ? 0 : op.kind == OP_GEMM ? 1 : op.kind == OP_DW ? 2 : op.kind == OP_FUSED ? 3 : 4;
         if (op_flops) op_flops[i] = op.flops_per_image * batch;
         if (op_bytes) op_bytes[i] = op.bytes_per_image * batch + op.weight_bytes;
     }

@@ -3,6 +3,7 @@
 Reference (paths relative to /root/reference/src/openpifpaf/):
   Shell.forward                       network/nets.py:35-48
   ShuffleNetV2K / InvertedResidualK   network/basenetworks.py:186-355
+  MobileNetV2 / MobileNetV3           network/basenetworks.py:407-458 (torchvision `features`)
   CompositeField4 (eval)              network/heads.py:330-378
 
 `plan_from_shell(shell)` walks a reference-style ``Shell`` (duck-typed: the
@@ -117,14 +118,110 @@ def _plan_from_resnet(shell):
     return plan
 
 
+# fused activation codes of the C ABI (include/pifpaf_b200.h)
+ACT_NONE, ACT_RELU, ACT_RELU6, ACT_HARDSWISH = 0, 1, 2, 3
+
+
+def _act_code(m):
+    for cls, code in ((torch.nn.ReLU, ACT_RELU), (torch.nn.ReLU6, ACT_RELU6), (torch.nn.Hardswish, ACT_HARDSWISH)):
+        if type(m) is cls:
+            return code
+    raise RuntimeError(f'unsupported module in the MobileNet backbone: {type(m).__name__} '
+                       '(only ReLU, ReLU6, Hardswish and squeeze-excitation with ReLU / Hardsigmoid)')
+
+
+def _conv_bn_act(seq):
+    """torchvision Conv2dNormActivation: Conv2d (bias-free), BatchNorm2d, optional activation."""
+    mods = list(seq.children())
+    if not (2 <= len(mods) <= 3 and isinstance(mods[0], torch.nn.Conv2d) and type(mods[1]) is torch.nn.BatchNorm2d):
+        raise RuntimeError('unsupported module in the MobileNet backbone: expected Conv2d, BatchNorm2d[, activation], '
+                           f'got {[type(m).__name__ for m in mods]}')
+    return mods[0], mods[1], (_act_code(mods[2]) if len(mods) == 3 else ACT_NONE)
+
+
+def _conv_entry(conv, bn, act):
+    if conv.dilation[0] != 1 or conv.dilation[1] != 1 or conv.kernel_size[0] != conv.kernel_size[1] or \
+            conv.stride[0] != conv.stride[1] or conv.padding[0] != conv.padding[1]:
+        raise RuntimeError('dilated / non-square MobileNet convolutions are not supported')
+    w, b = _fold(conv, bn)
+    return {'w': w, 'b': b, 'kernel': int(conv.kernel_size[0]), 'stride': int(conv.stride[0]),
+            'pad': int(conv.padding[0]), 'groups': int(conv.groups), 'act': act}
+
+
+def _plan_from_mobilenet(shell):
+    """basenetworks.py:407-458: `backbone` = torchvision MobileNetV2 / V3 `features` (the V3 stem stride set to 1 by
+    the reference is read from the module).  Stem Conv2dNormActivation, InvertedResidual blocks ([expand 1x1],
+    depthwise kxk, [SqueezeExcitation], linear 1x1 projection, residual when use_res_connect), last 1x1 conv."""
+    base = shell.base_net
+    feats = list(base.backbone.children())
+    if len(feats) < 3:
+        raise RuntimeError('unsupported MobileNet backbone: too few layers')
+    stem = _conv_entry(*_conv_bn_act(feats[0]))
+    if stem['groups'] != 1:
+        raise RuntimeError('unsupported MobileNet stem')
+    last = _conv_entry(*_conv_bn_act(feats[-1]))
+    if last['kernel'] != 1 or last['stride'] != 1 or last['groups'] != 1:
+        raise RuntimeError('unsupported MobileNet last layer: expected a 1x1 conv')
+    blocks = []
+    for blk in feats[1:-1]:
+        inner = getattr(blk, 'block', None)
+        if inner is None:
+            inner = getattr(blk, 'conv', None)              # torchvision MobileNetV2's InvertedResidual
+        if inner is None or not hasattr(blk, 'use_res_connect'):
+            raise RuntimeError(f'unsupported module in the MobileNet backbone: {type(blk).__name__}')
+        mods, units = list(inner.children()), []
+        i = 0
+        while i < len(mods):
+            m = mods[i]
+            if isinstance(m, torch.nn.Conv2d):             # MobileNetV2's projection: Conv2d, BatchNorm2d
+                if i + 1 >= len(mods) or type(mods[i + 1]) is not torch.nn.BatchNorm2d:
+                    raise RuntimeError('unsupported MobileNet block: a Conv2d without its BatchNorm2d')
+                units.append(_conv_entry(m, mods[i + 1], ACT_NONE))
+                i += 2
+            elif isinstance(m, torch.nn.Sequential):
+                units.append(_conv_entry(*_conv_bn_act(m)))
+                i += 1
+            elif hasattr(m, 'fc1') and hasattr(m, 'fc2'):  # torchvision SqueezeExcitation
+                if type(getattr(m, 'activation', None)) is not torch.nn.ReLU or \
+                        type(getattr(m, 'scale_activation', None)) is not torch.nn.Hardsigmoid:
+                    raise RuntimeError('unsupported module in the MobileNet backbone: squeeze-excitation '
+                                       'activations other than ReLU / Hardsigmoid')
+                units.append({'se': {'w1': m.fc1.weight.detach().float().cpu().numpy()[:, :, 0, 0],
+                                     'b1': m.fc1.bias.detach().float().cpu().numpy(),
+                                     'w2': m.fc2.weight.detach().float().cpu().numpy()[:, :, 0, 0],
+                                     'b2': m.fc2.bias.detach().float().cpu().numpy()}})
+                i += 1
+            else:
+                _act_code(m)                               # raises with the module's name
+                raise RuntimeError(f'unsupported module in the MobileNet backbone: {type(m).__name__}')
+        dw_i = [k for k, u in enumerate(units) if 'se' not in u and u['groups'] > 1]
+        if len(dw_i) != 1:
+            raise RuntimeError('unsupported MobileNet block: expected exactly one depthwise conv')
+        k = dw_i[0]
+        pre, dw, post = units[:k], units[k], units[k + 1:]
+        se = post.pop(0)['se'] if post and 'se' in post[0] else None
+        c_dw = dw['w'].shape[0]
+        if dw['groups'] != c_dw or dw['w'].shape[1] != 1 or dw['kernel'] not in (3, 5) or dw['stride'] not in (1, 2):
+            raise RuntimeError('unsupported MobileNet depthwise conv (3x3 / 5x5, stride 1 / 2 only)')
+        if len(pre) > 1 or len(post) != 1 or any(u['kernel'] != 1 or u['stride'] != 1 or u['groups'] != 1
+                                                 for u in pre + post) or post[0]['act'] != ACT_NONE:
+            raise RuntimeError('unsupported MobileNet block: expected [1x1], depthwise, [SE], linear 1x1')
+        blocks.append({'expand': pre[0] if pre else None, 'dw': dw, 'se': se, 'project': post[0],
+                       'residual': bool(blk.use_res_connect)})
+    return {'kind': 'mobilenet', 'input': stem, 'blocks': blocks, 'last': last, 'heads': _heads_plan(shell, base)}
+
+
 def plan_from_shell(shell):
-    """Extract a folded plan from a reference-style Shell (ShuffleNetV2K or Resnet base net)."""
+    """Extract a folded plan from a reference-style Shell (ShuffleNetV2K, Resnet, MobileNetV2 or MobileNetV3 base
+    net)."""
     base = shell.base_net
     if shell.training:
         raise RuntimeError('the Shell must be in eval() mode (BatchNorm is folded)')
     # network/nets.py:12-13,36-46: optional pre/post-processing hooks -- not lowered, so refuse them loudly
     if getattr(shell, 'process_input', None) is not None or getattr(shell, 'process_heads', None) is not None:
         raise RuntimeError('Shell.process_input / process_heads are not supported by the compiled forward')
+    if hasattr(base, 'backbone'):
+        return _plan_from_mobilenet(shell)
     for m in base.modules():
         # the kernels fuse max(x, 0); --shufflenetv2k-leaky-relu etc. would be folded wrongly
         if isinstance(m, (torch.nn.LeakyReLU, torch.nn.ELU, torch.nn.PReLU, torch.nn.SiLU, torch.nn.GELU,
@@ -258,6 +355,83 @@ def random_resnet_plan(base_name='resnet50', heads=((17, 1, 1, 1), (19, 1, 2, 2)
         b.reshape(nf, ncomp)[:, 1:1 + nconf] += np.float32(confidence_bias)
         plan['heads'].append({'w': w, 'b': b, 'n_fields': nf, 'n_comp': ncomp,
                               'ops': head_ops(nconf, nvec, nsc, (True,) * nvec), 'stride': 16})
+    return plan
+
+
+# torchvision.models.mobilenetv3._mobilenet_v3_conf / mobilenetv2 inverted_residual_setting (width 1.0):
+# (kernel, expanded channels, out channels, SE, activation code, stride) per block; stem channels, last conv channels
+MOBILENET_CONFIGS = {
+    'mobilenetv3large': (16, ACT_HARDSWISH, 960, 16, [
+        (3, 16, 16, False, 1, 1), (3, 64, 24, False, 1, 2), (3, 72, 24, False, 1, 1), (5, 72, 40, True, 1, 2),
+        (5, 120, 40, True, 1, 1), (5, 120, 40, True, 1, 1), (3, 240, 80, False, 3, 2), (3, 200, 80, False, 3, 1),
+        (3, 184, 80, False, 3, 1), (3, 184, 80, False, 3, 1), (3, 480, 112, True, 3, 1), (3, 672, 112, True, 3, 1),
+        (5, 672, 160, True, 3, 2), (5, 960, 160, True, 3, 1), (5, 960, 160, True, 3, 1)]),
+    'mobilenetv3small': (16, ACT_HARDSWISH, 576, 16, [
+        (3, 16, 16, True, 1, 2), (3, 72, 24, False, 1, 2), (3, 88, 24, False, 1, 1), (5, 96, 40, True, 3, 2),
+        (5, 240, 40, True, 3, 1), (5, 240, 40, True, 3, 1), (5, 120, 48, True, 3, 1), (5, 144, 48, True, 3, 1),
+        (5, 288, 96, True, 3, 2), (5, 576, 96, True, 3, 1), (5, 576, 96, True, 3, 1)]),
+}
+
+
+def _mobilenet_v2_blocks():
+    """(kernel, expanded, out, SE, act, stride) of torchvision's MobileNetV2 (expand ratio t of the block's INPUT)"""
+    out, cin = [], 32
+    for t, c, n, s in [(1, 16, 1, 1), (6, 24, 2, 2), (6, 32, 3, 2), (6, 64, 4, 2), (6, 96, 3, 1), (6, 160, 3, 2),
+                       (6, 320, 1, 1)]:
+        for i in range(n):
+            out.append((3, cin * t, c, False, ACT_RELU6, s if i == 0 else 1))
+            cin = c
+    return out
+
+
+MOBILENET_CONFIGS['mobilenetv2'] = (32, ACT_RELU6, 1280, 32, _mobilenet_v2_blocks())
+
+
+def _make_divisible(v, divisor=8):
+    """torchvision.models._utils._make_divisible (the squeeze channels of SqueezeExcitation)"""
+    new_v = max(divisor, int(v + divisor / 2) // divisor * divisor)
+    return new_v + divisor if new_v < 0.9 * v else new_v
+
+
+def random_mobilenet_plan(base_name='mobilenetv3large', heads=((17, 1, 1, 1), (19, 1, 2, 2)), seed=0,
+                          confidence_bias=-4.0):
+    """Random-init folded plan of the reference's MobileNetV2 / MobileNetV3 base networks (basenetworks.py:407-458;
+    V3 with the stem stride 1 the reference sets: output stride 16, V2: 32) -- the same dict layout
+    `_plan_from_mobilenet` extracts from a Shell.  He-scaled weights; the projection of a residual block gets half the
+    variance so that the sums keep the activation scale."""
+    c0, stem_act, c_last, stride, cfg = MOBILENET_CONFIGS[base_name]
+    rng = np.random.Generator(np.random.PCG64(seed))
+
+    def conv(cout, cin, k, stride_, act, groups=1, gain=2.0):
+        fan_in = cin // groups * k * k
+        w = rng.standard_normal((cout, cin // groups, k, k)).astype(np.float32) * np.float32(np.sqrt(gain / fan_in))
+        b = (rng.standard_normal(cout) * 0.05).astype(np.float32)
+        return {'w': w, 'b': b, 'kernel': k, 'stride': stride_, 'pad': (k - 1) // 2, 'groups': groups, 'act': act}
+
+    v3 = base_name.startswith('mobilenetv3')
+    plan = {'kind': 'mobilenet', 'input': conv(c0, 3, 3, 1 if v3 else 2, stem_act), 'blocks': [], 'heads': []}
+    cin = c0
+    for (k, ce, co, se, act, st) in cfg:
+        sq = _make_divisible(ce // 4)
+        blk = {'expand': conv(ce, cin, 1, 1, act) if ce != cin else None,
+               'dw': conv(ce, ce, k, st, act, groups=ce),
+               'se': None if not se else {
+                   'w1': (rng.standard_normal((sq, ce)) * np.sqrt(2.0 / ce)).astype(np.float32),
+                   'b1': (rng.standard_normal(sq) * 0.05).astype(np.float32),
+                   'w2': (rng.standard_normal((ce, sq)) * np.sqrt(1.0 / sq)).astype(np.float32),
+                   'b2': (rng.standard_normal(ce) * 0.05).astype(np.float32)},
+               'residual': st == 1 and cin == co}
+        blk['project'] = conv(co, ce, 1, 1, ACT_NONE, gain=1.0 if blk['residual'] else 2.0)
+        plan['blocks'].append(blk)
+        cin = co
+    plan['last'] = conv(c_last, cin, 1, 1, stem_act if v3 else ACT_RELU6)
+    for (nf, nconf, nvec, nsc) in heads:
+        ncomp = 1 + nconf + 2 * nvec + nsc
+        w = (rng.standard_normal((nf * ncomp, c_last)) * np.sqrt(1.0 / c_last)).astype(np.float32)
+        b = (rng.standard_normal(nf * ncomp) * 0.1).astype(np.float32)
+        b.reshape(nf, ncomp)[:, 1:1 + nconf] += np.float32(confidence_bias)
+        plan['heads'].append({'w': w, 'b': b, 'n_fields': nf, 'n_comp': ncomp,
+                              'ops': head_ops(nconf, nvec, nsc, (True,) * nvec), 'stride': stride})
     return plan
 
 
@@ -443,6 +617,8 @@ def build_ops(plan, in_h, in_w, layout=None, fuse_dw=None):
     {'input_conv', 'conv1x1', 'dwconv', 'heads'} whose fields are the C ABI arguments."""
     if plan.get('kind') == 'resnet':
         return _build_ops_resnet(plan, in_h, in_w)
+    if plan.get('kind') == 'mobilenet':
+        return _build_ops_mobilenet(plan, in_h, in_w)
     if plan.get('kind') == 'heads_only':
         # in_h x in_w is the FEATURE map here; the feature tensor is filled through CompiledNet.forward_features
         c_in = int(plan['c_in'])
@@ -679,6 +855,72 @@ def _build_ops_resnet(plan, in_h, in_w):
     return tensors, ops, {'block_outputs': block_outputs, 'feature': (cur, _Layout(c_cur, split=False))}
 
 
+def _build_ops_mobilenet(plan, in_h, in_w):
+    """torchvision InvertedResidual (eval): expand 1x1 GEMM (+ activation), depthwise kxk (+ activation), then the
+    linear projection -- a plain GEMM, a GEMM with the residual add fused (use_res_connect), or, behind a
+    squeeze-excitation, the 'se_conv1x1' op (pooled sums from the depthwise kernel, per-image projection weights)."""
+    tensors, ops = [], []
+
+    def tensor(h, w, c):
+        tensors.append((h, w, c))
+        return len(tensors) - 1
+
+    def out_hw(h, w, e):
+        return ((h + 2 * e['pad'] - e['kernel']) // e['stride'] + 1, (w + 2 * e['pad'] - e['kernel']) // e['stride'] + 1)
+
+    def conv1x1(tin, c_in, e, tout):
+        ops.append({'kind': 'conv1x1', 'in': tin, 'in_off': 0, 'k_cols': c_in, 'n_out': e['w'].shape[0],
+                    'w': _f32(e['w'].reshape(e['w'].shape[0], -1)), 'b': _f32(e['b']), 'relu': int(e['act']),
+                    'out': tout, 'out_off': 0, 'shuffle_src': -1, 'shuffle_off': 0})
+
+    inp = plan['input']
+    h, w = out_hw(in_h, in_w, inp)
+    c_cur = inp['w'].shape[0]
+    cur = tensor(h, w, pad16(c_cur))
+    ops.append({'kind': 'input_conv', 'in_h': in_h, 'in_w': in_w, 'kernel': inp['kernel'], 'stride': inp['stride'],
+                'pad': inp['pad'], 'c_out': c_cur, 'w': _f32(inp['w']), 'b': _f32(inp['b']), 'relu': int(inp['act']),
+                'out': cur})
+    block_outputs = []
+    for blk in plan['blocks']:
+        x_in, t_in, c_in = cur, cur, c_cur
+        if blk['expand'] is not None:
+            c_in = blk['expand']['w'].shape[0]
+            t_in = tensor(h, w, pad16(c_in))
+            conv1x1(cur, c_cur, blk['expand'], t_in)
+        dw = blk['dw']
+        ho, wo = out_hw(h, w, dw)
+        t_d = tensor(ho, wo, pad16(c_in))
+        k = dw['kernel']
+        ops.append({'kind': 'dwconv', 'in': t_in, 'in_off': 0, 'channels': c_in, 'kernel': k, 'stride': dw['stride'],
+                    'pad': dw['pad'], 'w': _f32(dw['w'].reshape(c_in, k * k)), 'b': _f32(dw['b']),
+                    'relu': int(dw['act']), 'out': t_d, 'out_off': 0})
+        pr = blk['project']
+        c_out = pr['w'].shape[0]
+        t_o = tensor(ho, wo, pad16(c_out))
+        res = x_in if blk['residual'] else -1
+        wp = _f32(pr['w'].reshape(c_out, c_in))
+        if blk['se'] is not None:
+            se = blk['se']
+            ops.append({'kind': 'se_conv1x1', 'in': t_d, 'channels': c_in, 'squeeze': se['w1'].shape[0],
+                        'fc1_w': _f32(se['w1']), 'fc1_b': _f32(se['b1']), 'fc2_w': _f32(se['w2']),
+                        'fc2_b': _f32(se['b2']), 'n_out': c_out, 'w': wp, 'b': _f32(pr['b']), 'out': t_o,
+                        'residual': res})
+        elif res >= 0:
+            ops.append({'kind': 'conv', 'in': t_d, 'in_off': 0, 'c_in': c_in, 'kernel': 1, 'stride': 1, 'pad': 0,
+                        'n_out': c_out, 'w': wp.reshape(c_out, c_in, 1, 1), 'b': _f32(pr['b']), 'relu': 0,
+                        'out': t_o, 'out_off': 0, 'residual': res, 'residual_off': 0})
+        else:
+            conv1x1(t_d, c_in, pr, t_o)
+        cur, c_cur, h, w = t_o, c_out, ho, wo
+        block_outputs.append((cur, _Layout(c_cur, split=False)))
+    last = plan['last']
+    c_last = last['w'].shape[0]
+    t_f = tensor(h, w, pad16(c_last))
+    conv1x1(cur, c_cur, last, t_f)
+    ops.append(_heads_op(plan['heads'], t_f, c_last))
+    return tensors, ops, {'block_outputs': block_outputs, 'feature': (t_f, _Layout(c_last, split=False))}
+
+
 class CompiledNet:
     """A plan compiled to libpifpaf_b200 ops for a fixed input size and maximum batch."""
 
@@ -755,6 +997,10 @@ class CompiledNet:
                 _lib.check(L.pifpaf_net_conv(H, o['in'], o['in_off'], o['c_in'], o['kernel'], o['stride'], o['pad'],
                                              o['n_out'], _ptr(o['w']), _ptr(o['b']), o['relu'], o['out'],
                                              o['out_off'], o['residual'], o['residual_off']))
+            elif o['kind'] == 'se_conv1x1':
+                _lib.check(L.pifpaf_net_se_conv1x1(H, o['in'], o['channels'], o['squeeze'], _ptr(o['fc1_w']),
+                                                   _ptr(o['fc1_b']), _ptr(o['fc2_w']), _ptr(o['fc2_b']), o['n_out'],
+                                                   _ptr(o['w']), _ptr(o['b']), o['out'], o['residual']))
             elif o['kind'] == 'dwconv':
                 _lib.check(L.pifpaf_net_dwconv(H, o['in'], o['in_off'], o['channels'], o['kernel'], o['stride'],
                                                o['pad'], _ptr(o['w']), _ptr(o['b']), o['relu'], o['out'], o['out_off']))
@@ -839,8 +1085,8 @@ class CompiledNet:
         return self._head_views(b)
 
     def forward_timed(self, image_batch, *, gemm_impl=0):
-        """Profiling pass: per-op (ms, kind, flops, bytes); kind 0 input conv, 1 tcgen05 GEMM, 2 depthwise,
-        3 fused depthwise -> GEMM."""
+        """Profiling pass: per library op (ms, kind, flops, bytes); kind 0 input conv, 1 tcgen05 GEMM, 2 depthwise,
+        3 fused depthwise -> GEMM, 4 squeeze-excitation (an 'se_conv1x1' op is two library ops: 4, then its GEMM)."""
         b, n = int(image_batch.shape[0]), self.num_ops
         ms = np.zeros((n,), dtype=np.float32)
         kind = np.zeros((n,), dtype=np.int32)
